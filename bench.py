@@ -4,11 +4,16 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [--gpus N] ...                # the reference algorithm on the host CPU cores
+    python bench.py --dump-outputs DIR                             # also write the last timed step's outputs
 
 One step = Trainer.global_step (src/defaults/trainer.py:106-138): forward, CrossEntropy, backward (weight
 gradients only for the APLA projection rows + head), data-parallel gradient mean, clip_grad_norm_(1.0), AdamW.
 Prints ONE JSON line (rank 0).  `value` = whole-job images/s with the batch resident in HBM; `e2e` = the same
 through the public API from pinned host buffers (H2D of the batch and D2H of the loss inside the timed region).
+Every timed leg runs exactly --steps steps; the >= 2.5 s sustained leg runs only with --sustained.
+
+Weights, APLA indices and batches are seeded, so the same arguments give the same inputs on every run and
+`--dump-outputs` of two builds can be compared array for array.
 """
 import argparse
 import json
@@ -134,6 +139,31 @@ def synthetic_batch(batch, img, n_classes, seed=1234, rank=0):
     import torch
     g = torch.Generator().manual_seed(seed + rank)
     return torch.randn(batch, 3, img, img, generator=g), torch.randint(0, n_classes, (batch,), generator=g)
+
+
+DUMP_MAX_BYTES = 64_000_000
+
+
+def host_outputs(named):
+    """{name: tensor} -> float32 CPU copies, taken right after the timed leg (later legs keep updating the state)."""
+    return {k: v.detach().float().cpu() for k, v in named.items()}
+
+
+def dump_outputs(path, arrays):
+    """Write {name: float32 CPU tensor} as <path>/<name>.npy.  When they hold more than DUMP_MAX_BYTES in all, every
+    array is replaced by a fixed, seeded sample of its flattened elements (a share proportional to its size; the same
+    positions on every run and every build), so that the dump stays within the limit."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    total = sum(t.numel() for t in arrays.values())
+    budget = (DUMP_MAX_BYTES - 4096 * len(arrays)) // 4          # values, leaving room for the .npy headers
+    for name, t in arrays.items():
+        if total > budget:
+            keep = max(1, t.numel() * budget // total)
+            pick = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t.flatten()[pick]
+        np.save(os.path.join(path, name + ".npy"), t.numpy())
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -360,6 +390,12 @@ def run_gpu(args):
     #  at least two untimed steps here, four for the two input slots of the end-to-end path)
     ms_step = timed(lambda: eng.step(images_dev, labels_dev), args.steps, max(2, args.warmup - 1))
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        # what the caller of eng.step() holds after the last timed step: loss, logits, trainable parameters and their
+        # (clipped, rank-averaged) gradients
+        outputs = host_outputs(dict(loss=eng.loss.reshape(1), logits=eng.logits,
+                                    **{"param." + k: v for k, v in eng.named_params().items()},
+                                    **{"grad." + k: v for k, v in eng.named_grads().items()}))
     ms_e2e = timed(lambda: eng.step_from_host(images_pin, labels_pin), args.steps, max(4, args.warmup // 2))
     loss = eng.drain()
     if loss is None:
@@ -442,6 +478,8 @@ def run_gpu(args):
                 # BASELINE.json configs[0] / BASELINE.md section 3: the reference path on C1 exactly (ViT-S/16, r = 32, batch 8)
                 c1, _ = cpu_reference_steps(steps=6, warmup=2, batch=8, w=C1)
                 line["cpu_baseline_c1"] = c1
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -551,6 +589,11 @@ def run_ssl(args):
         b = {k: (v.to(dev, non_blocking=True) if torch.is_tensor(v) else v) for k, v in batch_pin.items()}
         return float(step(b))                                         # loss read back to the host every step
 
+    last = {}
+
+    def timed_step():
+        last["loss"] = step(batch_dev).detach()
+
     sampler = ClockSampler(local) if rank == 0 else None
     step(batch_dev)
     n0 = LIB.load().apla_launch_count()
@@ -558,9 +601,15 @@ def run_ssl(args):
     launches_per_step = int(LIB.load().apla_launch_count() - n0)
     if sampler:
         sampler.start()
-    ms_step = timed(lambda: step(batch_dev), args.steps, max(1, args.warmup - 2))
+    ms_step = timed(timed_step, args.steps, max(1, args.warmup - 2))
     clocks = sampler.stop() if sampler else None
-    ms_e2e = timed(step_e2e, max(3, args.steps // 2), 1)
+    if args.dump_outputs and rank == 0:
+        # what the caller of the step holds after the last timed step: the loss, the student's trainable parameters
+        # after AdamW and their clipped gradients
+        named = [(n, p) for n, p in model.student.named_parameters() if p.requires_grad]
+        outputs = host_outputs(dict(loss=last["loss"].reshape(1), **{"param." + n: p for n, p in named},
+                                    **{"grad." + n: p.grad for n, p in named}))
+    ms_e2e = timed(step_e2e, args.steps, 1)
     loss = float(step(batch_dev))
     if rank == 0:
         peaks = load_peaks()
@@ -594,6 +643,8 @@ def run_ssl(args):
             masked_patches=int(batch_host["mask_indices_list"].shape[0]),
             trainable_params=sum(p.numel() for p in trainable), peak_hbm_gb=round(torch.cuda.max_memory_allocated() / 1e9, 1),
             gpu_launches=launches_per_step * args.steps, gpu_launches_per_step=launches_per_step, clocks=clocks)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -603,7 +654,7 @@ def run_ssl(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of every timed leg")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=0, help="per-GPU batch override (default: the workload's 64)")
@@ -612,11 +663,20 @@ def main():
                     help="c2 = BASELINE.json configs[1] (the metric's configuration, default); c3 / c5 / vitl: other shapes "
                          "through the engine; c4 = configs[3], the DINOv2 self-supervised step (module-level path)")
     ap.add_argument("--no-c3", action="store_true", help="skip the nested configs[2] (partial_size 768) leg of the c2 line")
-    ap.add_argument("--no-sustained", dest="sustained", action="store_false",
-                    help="skip the >= 2.5 s sustained leg (roofline.step.sustained_*)")
+    ap.add_argument("--sustained", action="store_true",
+                    help="add a leg that runs the step for >= 2.5 s, however many steps that takes (roofline.step.sustained_*)")
+    ap.add_argument("--no-sustained", dest="sustained", action="store_false", help="no sustained leg (the default)")
     ap.add_argument("--per-term-losses", action="store_true",
                     help="c4: the reference's call structure (one loss-class call per term) instead of the fused objective")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (loss, logits, trainable "
+                         "parameters and gradients) as DIR/<name>.npy, float32, at most 64 MB in all (larger outputs: "
+                         "a fixed, seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this project's CUDA path; --impl reference has none")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "c4":
