@@ -8,7 +8,9 @@ tensor-core GEMMs unless the caller wraps it in autocast.  `fuse_apla_blocks(mod
 is an `APLA_Attention` for a `FusedAplaBlock` that holds the SAME sub-modules under the SAME names (state-dict keys and
 checkpoints unchanged) and runs forward and backward through the kernels the step engine uses:
 
-  (two native calls per block and step: `apla_block_fwd`, `apla_block_bwd`, csrc/block.cu)
+  (two native calls per block and step: `apla_block_fwd`, `apla_block_bwd`, csrc/block.cu; when autograd would record
+  nothing -- under torch.no_grad(), or with neither the input nor proj_weight1 / proj_bias1 requiring grad -- the forward
+  is `apla_block_fwd_infer` instead: same output bit for bit, no saved tensors, no GELU derivative written)
   forward   LN1 -> qkv GEMM -> fused attention (saves log-sum-exp) -> proj GEMM (+bias, xLayerScale, +residual, fp32)
             -> LN2 -> fc1 GEMM (+bias, GELU, saves gelu' in fp16) -> fc2 GEMM (+bias, xLayerScale, +residual, fp32)
   backward  LayerScale+cast -> fc2 dgrad x gelu' -> fc1 dgrad -> LN2' (+residual grad, xLayerScale, APLA column gather)
@@ -42,30 +44,35 @@ from .appla_attn import APLA_Attention, _pad64
 _CHAIN = os.environ.get("APLA_BLOCK_CHAIN", "1") != "0"      # hand bf16(gamma2 * dx) from block to block in backward
 
 
+def _fwd_setup(blk, x, cu_seqlens, seqlens):
+    """Native weights, fp32 input rows, geometry and the buffers both forwards write:
+    -> (nat, x_in, T, num_seqs, max_len, (x_mid, x_out, qkv, ao, lse, ln_tmp, gelu_tmp))."""
+    at = blk.attn
+    nat = blk._native(x.device)
+    D, H, Hd = at.dim, at.num_heads, blk.mlp.fc1.out_features
+    x_in = x.reshape(-1, D).to(torch.float32).contiguous()
+    T = x_in.shape[0]
+    if cu_seqlens is None:
+        num_seqs, max_len = (x.shape[0], x.shape[1]) if x.dim() == 3 else (1, T)
+    else:
+        num_seqs, max_len = len(seqlens), max(seqlens)
+    dev, bf, f32 = x.device, torch.bfloat16, torch.float32
+    bufs = (torch.empty(T, D, device=dev, dtype=f32), torch.empty(T, D, device=dev, dtype=f32),
+            torch.empty(T, 3 * D, device=dev, dtype=bf), torch.empty(T, D, device=dev, dtype=bf),
+            torch.empty(T, H, device=dev, dtype=f32), torch.empty(T, D, device=dev, dtype=bf),
+            torch.empty(T, Hd, device=dev, dtype=bf))
+    return nat, x_in, T, num_seqs, max_len, bufs
+
+
 class _AplaBlockFn(torch.autograd.Function):
     """One native call per direction (`apla_block_fwd` / `apla_block_bwd`, csrc/block.cu): 7 + up to 13 kernel launches
     with no Python between them."""
 
     @staticmethod
     def forward(ctx, x, w1, b1, blk, cu_seqlens, seqlens):
-        at = blk.attn
-        nat = blk._native(x.device)
-        D, H, Hd = at.dim, at.num_heads, blk.mlp.fc1.out_features
-        x_in = x.reshape(-1, D).to(torch.float32).contiguous()
-        T = x_in.shape[0]
-        if cu_seqlens is None:
-            num_seqs, max_len = (x.shape[0], x.shape[1]) if x.dim() == 3 else (1, T)
-        else:
-            num_seqs, max_len = len(seqlens), max(seqlens)
-        dev, bf, f32 = x.device, torch.bfloat16, torch.float32
-        x_mid = torch.empty(T, D, device=dev, dtype=f32)
-        x_out = torch.empty(T, D, device=dev, dtype=f32)
-        qkv = torch.empty(T, 3 * D, device=dev, dtype=bf)
-        ao = torch.empty(T, D, device=dev, dtype=bf)
-        lse = torch.empty(T, H, device=dev, dtype=f32)
-        dgelu = torch.empty(T, Hd, device=dev, dtype=torch.float16)
-        ln_tmp = torch.empty(T, D, device=dev, dtype=bf)
-        gelu_tmp = torch.empty(T, Hd, device=dev, dtype=bf)
+        nat, x_in, T, num_seqs, max_len, (x_mid, x_out, qkv, ao, lse, ln_tmp, gelu_tmp) = _fwd_setup(blk, x, cu_seqlens,
+                                                                                                    seqlens)
+        dgelu = torch.empty(T, blk.mlp.fc1.out_features, device=x.device, dtype=torch.float16)
         LIB.call("apla_block_fwd", ctypes.addressof(nat), ptr(x_in), ptr(x_mid), ptr(x_out), ptr(ln_tmp), ptr(qkv), ptr(ao),
                  ptr(lse), ptr(dgelu), ptr(gelu_tmp), ptr(cu_seqlens), num_seqs, max_len, T, stream())
         ctx.blk, ctx.nat, ctx.refs = blk, nat, blk._nat_refs      # the struct points into these tensors
@@ -232,7 +239,18 @@ class FusedAplaBlock(nn.Module):
 
     def _run_fused(self, x, cu=None, seqlens=None):
         at = self.attn
+        if not torch.is_grad_enabled() or not (x.requires_grad or at.proj_weight1.requires_grad
+                                                or at.proj_bias1.requires_grad):
+            return self._run_infer(x, cu, seqlens)      # autograd would record nothing: keep nothing for backward
         return _AplaBlockFn.apply(x, at.proj_weight1, at.proj_bias1, self, cu, seqlens)
+
+    def _run_infer(self, x, cu, seqlens):
+        """`apla_block_fwd_infer`: the forward of _AplaBlockFn, bit for bit, without its saved tensors (lse is scratch,
+        fc1 writes no GELU derivative).  x_out is a buffer of its own: x_in may be the caller's tensor."""
+        nat, x_in, T, num_seqs, max_len, (x_mid, x_out, qkv, ao, lse, ln_tmp, gelu_tmp) = _fwd_setup(self, x, cu, seqlens)
+        LIB.call("apla_block_fwd_infer", ctypes.addressof(nat), ptr(x_in), ptr(x_mid), ptr(x_out), ptr(ln_tmp), ptr(qkv),
+                 ptr(ao), ptr(lse), ptr(gelu_tmp), ptr(cu), num_seqs, max_len, T, stream())
+        return x_out.view(x.shape).to(x.dtype)
 
     def forward(self, x_or_x_list, return_attention: bool = False, return_intermediate: bool = False):
         """`[B,N,D]` -> `[B,N,D]` (vit.py:279-288) or list of `[b_i,N_i,D]` -> list (dinov2 block.py:274-288)."""

@@ -47,6 +47,27 @@ int apla_block_fwd(const apla_block_weights* w, const float* x_in, float* x_mid,
   return gemm_tn(EPI_RESID, gelu_tmp, w->wfc2, T, D, Hd, Hd, Hd, x_out, nullptr, w->bfc2, w->g2, x_mid, D, s, 0);
 }
 
+int apla_block_fwd_infer(const apla_block_weights* w, const float* x_in, float* x_mid, float* x_out, void* ln_tmp,
+                         void* qkv, void* ao, float* lse_tmp, void* gelu_tmp, const int32_t* cu_seqlens, int num_seqs,
+                         int max_seqlen, int T, apla_stream_t stream) {
+  if (int rc = check_weights(w, "apla_block_fwd_infer")) return rc;
+  APLA_CHECK(T > 0 && num_seqs > 0 && max_seqlen > 0, "apla_block_fwd_infer: empty problem");
+  APLA_CHECK(x_in && x_mid && x_out && ln_tmp && qkv && ao && lse_tmp && gelu_tmp, "apla_block_fwd_infer: null buffer");
+  APLA_CHECK(x_mid != x_in && x_mid != x_out, "apla_block_fwd_infer: x_mid may not alias x_in or x_out");
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  const int D = w->D, Hd = w->hidden;
+  // apla_block_fwd's sequence; fc1 writes gelu(h) only.  x_in is last read by the projection, so x_out may alias it.
+  if (int rc = layernorm_fwd(x_in, D, w->ln1w, w->ln1b, ln_tmp, D, T, D, w->eps1, s)) return rc;
+  if (int rc = gemm_tn(EPI_BIAS, ln_tmp, w->wqkv, T, 3 * D, D, D, D, qkv, nullptr, w->bqkv, nullptr, nullptr, 3 * D, s, 0))
+    return rc;
+  if (int rc = attn_fwd(qkv, ao, lse_tmp, cu_seqlens, num_seqs, max_seqlen, T, w->H, w->scale, s)) return rc;
+  if (int rc = gemm_tn(EPI_RESID, ao, w->wproj, T, D, D, D, D, x_mid, nullptr, w->bproj, w->g1, x_in, D, s, 0)) return rc;
+  if (int rc = layernorm_fwd(x_mid, D, w->ln2w, w->ln2b, ln_tmp, D, T, D, w->eps2, s)) return rc;
+  if (int rc = gemm_tn(EPI_BIAS_GELU_G, ln_tmp, w->wfc1, T, Hd, D, D, D, gelu_tmp, nullptr, w->bfc1, nullptr, nullptr, Hd, s, 0))
+    return rc;
+  return gemm_tn(EPI_RESID, gelu_tmp, w->wfc2, T, D, Hd, Hd, Hd, x_out, nullptr, w->bfc2, w->g2, x_mid, D, s, 0);
+}
+
 int apla_block_bwd(const apla_block_weights* w, const float* dx_out, const float* x_in, const float* x_mid,
                    const void* qkv, const void* ao, const float* lse, const void* dgelu, float* dx_mid, float* dx_in,
                    void* dyb, void* dh, void* dln, void* dsub, void* d_ao, float* delta, void* dqkv, float* dw1,

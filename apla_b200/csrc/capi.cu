@@ -59,6 +59,14 @@ int apla_gemm_bias_gelu_dgelu_fwd(const void* A, int lda, const void* W, int ldw
                                   int ldo, int M, int N, int K, apla_stream_t stream) {
   return gemm_tn(EPI_BIAS_GELU_D, A, W, M, N, K, lda, ldw, dgelu, g, bias, nullptr, nullptr, ldo, S(stream), 0);
 }
+int apla_gemm_bias_gelu_only_fwd(const void* A, int lda, const void* W, int ldw, const float* bias, void* g, int ldo,
+                                 int M, int N, int K, apla_stream_t stream) {
+  if (!A || !W || !g) {
+    set_error("apla_gemm_bias_gelu_only_fwd: null A, W or g");
+    return 1;
+  }
+  return gemm_tn(EPI_BIAS_GELU_G, A, W, M, N, K, lda, ldw, g, nullptr, bias, nullptr, nullptr, ldo, S(stream), 0);
+}
 int apla_gemm_dgrad_mul(const void* dY, int ldy, const void* Wt, int ldwt, const void* mul, void* dH, int ldh, int M,
                         int K_in, int N_out, apla_stream_t stream) {
   return gemm_tn(EPI_MUL_F16, dY, Wt, M, K_in, N_out, ldy, ldwt, dH, nullptr, nullptr, nullptr, mul, ldh, S(stream), 0);
@@ -130,6 +138,9 @@ int apla_head_fwd(const void* xn, const float* W, const float* bias, float* logi
 int apla_cross_entropy(const float* logits, const int64_t* labels, float* dlogits, float* loss, int B, int C,
                        float grad_scale, float loss_scale, apla_stream_t stream) {
   return cross_entropy(logits, labels, dlogits, loss, B, C, grad_scale, loss_scale, S(stream));
+}
+int apla_eval_accumulate(const float* logits, const int64_t* labels, int B, int C, float* acc, apla_stream_t stream) {
+  return eval_accumulate(logits, labels, B, C, acc, S(stream));
 }
 int apla_head_bwd(const float* dlogits, const void* xn, const float* W, float* dW, float* db, void* dxn, int B, int D,
                   int C, apla_stream_t stream) {

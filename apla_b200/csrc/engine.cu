@@ -50,6 +50,8 @@ struct Engine {
   // side_wgrad = number of dsub slots the host allocated (2 enables the side stream for partial_size < dim; the
   // full-rows path reads dxb and needs none).
   int side_wgrad = 0;
+  // evaluation forward (apla_engine_infer): images per call at most, set by option "infer_batch"; 0 = no workspace
+  int infer_cap = 0;
   cudaStream_t side = nullptr;
   std::vector<cudaEvent_t> ev_fork, ev_done;
   ~Engine() {
@@ -94,6 +96,12 @@ static const char* kGlobalNames[] = {
 // optional global buffers (not checked by check_ready): "hyper" = float[3] {lr, 1 - beta1^t, sqrt(1 - beta2^t)} read by
 // the AdamW kernel instead of its launch arguments, so that a captured step can be replayed with new values
 static const char* kOptionalNames[] = {"hyper"};
+
+// evaluation workspace (apla_engine_infer), sized for infer_cap images of N tokens; none of it is used by the step.
+// "infer_x" holds two fp32 [cap*N, D] residual buffers: the block input (overwritten by the block output) and the stream
+// after the attention branch -- two buffers whatever the depth.
+static const char* kInferNames[] = {"infer_x", "infer_ln", "infer_qkv", "infer_ao", "infer_lse", "infer_gelu",
+                                    "infer_patches", "infer_pe_out", "infer_cls_ln"};
 
 static int check_ready(Engine* e) {
   for (const char* n : kGlobalNames) {
@@ -197,6 +205,77 @@ static int engine_forward(Engine* e, const float* images, const int64_t* labels,
       return rc;
   }
   return 0;
+}
+
+static int check_infer_ready(Engine* e, int n_img) {
+  APLA_CHECK(e->infer_cap > 0, "apla_engine_infer: no evaluation workspace (option 'infer_batch' is 0)");
+  APLA_CHECK(n_img >= 1 && n_img <= e->infer_cap, "apla_engine_infer: n_img=%d outside [1, %d]", n_img, e->infer_cap);
+  for (const char* n : kInferNames)
+    APLA_CHECK(e->g.count(n) && e->g[n] != nullptr, "apla_engine_infer: workspace '%s' was not set", n);
+  for (const char* n : {"wpe", "bpe", "cls", "pos", "lnfw", "lnfb", "params"})
+    APLA_CHECK(e->g.count(n) && e->g[n] != nullptr, "apla_engine_infer: buffer '%s' was not set", n);
+  for (int l = 0; l < e->L; ++l) {
+    const BlockPtrs& b = e->blk[l];
+    APLA_CHECK(b.wqkv && b.wfc1 && b.wfc2 && b.wproj && b.bproj && b.bfc1 && b.bfc2 && b.ln1w && b.ln1b && b.ln2w && b.ln2b,
+               "apla_engine_infer: block %d has unset weights", l);
+  }
+  return 0;
+}
+
+// Classifier.forward (models.py:81-92) for n_img images with the engine's current weights, in the launch sequence of
+// engine_forward (same kernels, same gemm_resid_ln pairing, same CLS-only last block), but over its own workspace and
+// with the forward-only fc1 epilogue: nothing is kept for a backward pass.
+static int engine_infer(Engine* e, const float* images, int n_img, float* logits, void* emb, cudaStream_t s) {
+  if (int rc = check_infer_ready(e, n_img)) return rc;
+  const int B = n_img, N = e->N, D = e->D, L = e->L, Hd = e->hidden, T = B * N;
+  float* xa = e->get<float>("infer_x");                       // block input, then block output
+  float* xb = xa + size_t(e->infer_cap) * N * D;              // after the attention branch
+  void* ln = e->get<void>("infer_ln");
+  void* qkv = e->get<void>("infer_qkv");
+  void* ao = e->get<void>("infer_ao");
+  float* lse = e->get<float>("infer_lse");
+  void* gelu = e->get<void>("infer_gelu");
+  void* patches = e->get<void>("infer_patches");
+  void* pe_out = e->get<void>("infer_pe_out");
+  void* cls_ln = emb ? emb : e->get<void>("infer_cls_ln");
+  const Arena ar = arena_of(e);
+  const float* params = e->get<float>("params");
+
+  if (int rc = patchify(images, patches, B, e->img, e->patch, e->kpad, s)) return rc;
+  if (int rc = gemm_tn(EPI_BIAS, patches, e->get<void>("wpe"), B * e->P, D, e->kpad, e->kpad, e->kpad, pe_out, nullptr,
+                       e->get<float>("bpe"), nullptr, nullptr, D, s, 0))
+    return rc;
+  if (int rc = assemble_tokens(pe_out, e->get<float>("cls"), e->get<float>("pos"), xa, B, e->P, D, s)) return rc;
+  for (int l = 0; l < L; ++l) {
+    const BlockPtrs& b = e->blk[l];
+    if (l == 0) {
+      if (int rc = layernorm_fwd(xa, D, b.ln1w, b.ln1b, ln, D, T, D, e->eps, s)) return rc;
+    }
+    if (int rc = gemm_tn(EPI_BIAS, ln, b.wqkv, T, 3 * D, D, D, D, qkv, nullptr, b.bqkv, nullptr, nullptr, 3 * D, s, 0))
+      return rc;
+    const bool cls = e->cls_last && l == L - 1;
+    if (cls && e->cls_last >= 2) {
+      if (int rc = attn_cls_fwd(qkv, ao, lse, B, N, e->H, e->scale, s)) return rc;
+    } else {
+      if (int rc = attn_fwd(qkv, ao, lse, nullptr, B, N, T, e->H, e->scale, s)) return rc;
+    }
+    const int R = cls ? B : T;
+    const int sD = cls ? N * D : D, sH = cls ? N * Hd : Hd;
+    if (int rc = gemm_resid_ln(ao, b.wproj, R, D, D, sD, D, xb, b.bproj, b.g1, xa, sD, b.ln2w, b.ln2b, ln, sD, e->eps, s))
+      return rc;
+    if (int rc = gemm_tn(EPI_BIAS_GELU_G, ln, b.wfc1, R, Hd, D, sD, D, gelu, nullptr, b.bfc1, nullptr, nullptr, sH, s, 0))
+      return rc;
+    if (l + 1 < L) {
+      const BlockPtrs& nb = e->blk[l + 1];
+      if (int rc = gemm_resid_ln(gelu, b.wfc2, R, D, Hd, sH, Hd, xa, b.bfc2, b.g2, xb, sD, nb.ln1w, nb.ln1b, ln, sD, e->eps, s))
+        return rc;
+    } else {
+      if (int rc = gemm_tn(EPI_RESID, gelu, b.wfc2, R, D, Hd, sH, Hd, xa, nullptr, b.bfc2, b.g2, xb, sD, s, 0)) return rc;
+    }
+  }
+  if (int rc = layernorm_fwd(xa, int64_t(N) * D, e->get<float>("lnfw"), e->get<float>("lnfb"), cls_ln, D, B, D, e->eps, s))
+    return rc;
+  return head_fwd(cls_ln, params + ar.fcw, params + ar.fcb, logits, B, D, e->C, s);
 }
 
 static int engine_backward(Engine* e, int l_from, int l_to, cudaStream_t s) {
@@ -370,6 +449,7 @@ int apla_engine_set_ptr(apla_engine_t h, const char* name, int block, void* p) {
     bool known = false;
     for (const char* k : kGlobalNames) known |= (n == k);
     for (const char* k : kOptionalNames) known |= (n == k);
+    for (const char* k : kInferNames) known |= (n == k);
     APLA_CHECK(known, "apla_engine_set_ptr: unknown global buffer '%s'", name);
     e->g[n] = p;
     return 0;
@@ -396,6 +476,11 @@ int apla_engine_set_option(apla_engine_t h, const char* name, int value) {
     e->cls_last = value < 0 ? 0 : (value > 2 ? 2 : value);
     return 0;
   }
+  if (std::string(name) == "infer_batch") {   // capacity of the evaluation workspace in images (0 = none)
+    APLA_CHECK(value >= 0, "apla_engine_set_option: infer_batch=%d is negative", value);
+    e->infer_cap = value;
+    return 0;
+  }
   if (std::string(name) == "side_wgrad") {   // 0 = off, 1 = on for partial_size == dim, 2 = on, "dsub" holds two slots
     e->side_wgrad = value < 0 ? 0 : (value > 2 ? 2 : value);
     return 0;
@@ -418,6 +503,11 @@ int apla_engine_forward(apla_engine_t h, const float* images, const int64_t* lab
   Engine* e = reinterpret_cast<Engine*>(h);
   APLA_CHECK(e != nullptr && images != nullptr, "apla_engine_forward: null handle or images");
   return engine_forward(e, images, labels, loss_scale, grad_scale, reinterpret_cast<cudaStream_t>(stream));
+}
+int apla_engine_infer(apla_engine_t h, const float* images, int n_img, float* logits, void* emb, apla_stream_t stream) {
+  Engine* e = reinterpret_cast<Engine*>(h);
+  APLA_CHECK(e != nullptr && images != nullptr && logits != nullptr, "apla_engine_infer: null handle, images or logits");
+  return engine_infer(e, images, n_img, logits, emb, reinterpret_cast<cudaStream_t>(stream));
 }
 int apla_engine_backward(apla_engine_t h, int block_from, int block_to, apla_stream_t stream) {
   Engine* e = reinterpret_cast<Engine*>(h);

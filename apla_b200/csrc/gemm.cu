@@ -364,7 +364,7 @@ int gemm_tn(int epi, const void* A, const void* B, int M, int N, int K, int lda,
              "gemm_tn: this epilogue needs aux");
   APLA_CHECK(epi != EPI_MUL_F16 || aux != nullptr, "gemm_tn: EPI_MUL_F16 needs the fp16 multiplier in aux");
   APLA_CHECK(epi != EPI_BIAS_GELU_D || out2 != nullptr, "gemm_tn: EPI_BIAS_GELU_D needs out2");
-  if (epi == EPI_DELTA || epi == EPI_BIAS_GELU_D || epi == EPI_MUL_F16 || epi == EPI_RED) {   // 2-CTA kernel only
+  if (epi == EPI_DELTA || epi == EPI_BIAS_GELU_D || epi == EPI_BIAS_GELU_G || epi == EPI_MUL_F16 || epi == EPI_RED) {   // 2-CTA kernel only
     APLA_CHECK(epi != EPI_DELTA || (out2 != nullptr && N % 64 == 0),
                "gemm_tn: EPI_DELTA needs the delta buffer in out2 and N %% 64 == 0");
     int bn = bn_override;

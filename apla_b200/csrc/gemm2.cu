@@ -13,6 +13,8 @@
 //               to global memory, 32 rows per instruction, and was LSU-wavefront-bound in every fused epilogue).
 // Epilogues: see kernels.cuh / gemm.cu header (EPI_BIAS, EPI_BIAS_GELU, EPI_RESID, EPI_GELU_BWD), plus
 //   EPI_BIAS_GELU_D  h = acc + bias[n] (fp32, not stored);  out_f16 = gelu_erf'(h);  out2_bf16 = gelu_erf(h)
+//   EPI_BIAS_GELU_G  out_bf16 = gelu_erf(acc + bias[n]), bit-identical to out2 of EPI_BIAS_GELU_D: the forward-only
+//                    fc1, with the EPI_BIAS data path (one 128-byte staging row and one TMA store per 64-column chunk)
 //   EPI_MUL_F16      out_bf16 = acc * aux_f16[m,n]   (fc2 dgrad times the saved GELU derivative)
 //   EPI_RESID_LN     EPI_RESID, then the LayerNorm that reads the new residual stream: the CTA that completes the LAST
 //                    column tile of a 128-row slab (a self-resetting arrival counter per slab in global memory)
@@ -239,6 +241,8 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ 
     constexpr bool kAux = (EPI == EPI_RESID || kLN || EPI == EPI_GELU_BWD || EPI == EPI_DELTA || EPI == EPI_MUL_F16);
     constexpr bool kBias = (EPI != EPI_GELU_BWD && EPI != EPI_DELTA && EPI != EPI_MUL_F16);
     constexpr bool kTwoOut = (EPI == EPI_BIAS_GELU || EPI == EPI_BIAS_GELU_D);
+    // the GELU epilogues in packed fp32 add the bias inside gelu_erf_both_x2, not to the accumulator beforehand
+    constexpr bool kGeluX2 = (EPI == EPI_BIAS_GELU_D || EPI == EPI_BIAS_GELU_G);
     // columns per chunk: one 128-byte staging row, except the two-output GELU epilogue which packs a 64-byte row of
     // each output (h | g) into one 4 KB buffer (64B swizzle) so that chunks can still ping-pong between buffers
     constexpr int CW = (kF32 || kTwoOut) ? 32 : 64;
@@ -315,7 +319,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ 
       // thread as soon as the LAST sub-load has landed in registers -- not after the math and stores of the tile.
       uint32_t v[2][32];
       [[maybe_unused]] float4 bb[8];   // bias of the NEXT sub-load, fetched right after the current one is consumed
-      if constexpr (EPI == EPI_BIAS_GELU_D) {
+      if constexpr (kGeluX2) {
 #pragma unroll
         for (int i = 0; i < 8; ++i) bb[i] = make_float4(0.f, 0.f, 0.f, 0.f);   // stays zero when there is no bias
       }
@@ -375,9 +379,9 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ 
 #pragma unroll
           for (int i = 0; i < 32; ++i) x[i] = __uint_as_float(v[idx & 1][i]);
           const int col = col0 + s * 32;
-          [[maybe_unused]] float bv[32];   // EPI_BIAS_GELU_D adds the bias inside its packed-fp32 math
+          [[maybe_unused]] float bv[32];   // the GELU epilogues add the bias inside their packed-fp32 math
           if constexpr (kBias) {
-            if constexpr (EPI == EPI_BIAS_GELU_D) {
+            if constexpr (kGeluX2) {
 #pragma unroll
               for (int i = 0; i < 8; ++i) {
                 const float4 t4 = bb[i];
@@ -391,7 +395,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ 
                   const float4 t4 = __ldg(reinterpret_cast<const float4*>(bias + col) + i);
                   x[4 * i] += t4.x; x[4 * i + 1] += t4.y; x[4 * i + 2] += t4.z; x[4 * i + 3] += t4.w;
                 }
-              } else if constexpr (EPI != EPI_BIAS_GELU_D) {
+              } else if constexpr (!kGeluX2) {
 #pragma unroll
                 for (int i = 0; i < 8; ++i) {
                   const float4 t4 = bb[i];
@@ -436,6 +440,17 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ 
               const uint32_t off = lane * 64 + ((c ^ ((lane >> 1) & 3)) << 4);   // 64B-swizzled row of 32 x 2 bytes
               sts128(buf + off, dd[0], dd[1], dd[2], dd[3]);
               sts128(buf + kStgBuf / 2 + off, g[0], g[1], g[2], g[3]);
+            }
+          } else if constexpr (EPI == EPI_BIAS_GELU_G) {
+            // the same packed-fp32 evaluation as EPI_BIAS_GELU_D, so that g is bit-identical to the training forward's;
+            // the instructions that only feed the derivative are dead and the compiler drops them
+#pragma unroll
+            for (int c = 0; c < 4; ++c) {
+              uint32_t g[4], dd;
+#pragma unroll
+              for (int t = 0; t < 4; ++t)
+                gelu_erf_both_x2(x[8 * c + 2 * t], x[8 * c + 2 * t + 1], bv[8 * c + 2 * t], bv[8 * c + 2 * t + 1], g[t], dd);
+              sts128(stg_addr(buf, lane, 4 * s + c), g[0], g[1], g[2], g[3]);
             }
           } else if constexpr (EPI == EPI_MUL_F16) {
 #pragma unroll
@@ -629,6 +644,8 @@ int gemm2_tn(int epi, const void* A, const void* B, int M, int N, int K, int lda
       return g2::dispatch<EPI_RED>(A, B, M, N, K, lda, ldb, out, out2, bias, gamma, aux, ldo, stream, bn);
     case EPI_MUL_F16:
       return g2::dispatch<EPI_MUL_F16>(A, B, M, N, K, lda, ldb, out, out2, bias, gamma, aux, ldo, stream, bn);
+    case EPI_BIAS_GELU_G:
+      return g2::dispatch<EPI_BIAS_GELU_G>(A, B, M, N, K, lda, ldb, out, out2, bias, gamma, aux, ldo, stream, bn);
   }
   set_error("gemm2_tn: unknown epilogue %d", epi);
   return 1;

@@ -63,6 +63,57 @@ __global__ void ce_kernel(const float* __restrict__ logits, const int64_t* __res
   if (threadIdx.x == 0) atomicAdd(loss, (lse - lr[y]) * loss_scale);
 }
 
+// Evaluation sums over one batch, one CTA: acc[0] += sum_b CE_b (the row softmax of ce_kernel, one warp per row),
+// acc[1] += #{b : argmax_c logits[b,c] == labels[b]} with the first maximum winning, as torch.argmax picks it.  Each warp
+// walks its rows in order and the warps' partial sums are added in warp order: the result does not depend on timing.
+// A label outside [0, C) makes the loss NaN rather than reading outside the row.
+constexpr int kEvalThreads = 512;
+__global__ void __launch_bounds__(kEvalThreads) eval_acc_kernel(const float* __restrict__ logits,
+                                                               const int64_t* __restrict__ labels, int B, int C,
+                                                               float* __restrict__ acc) {
+  constexpr int kWarps = kEvalThreads / 32;
+  __shared__ float ce_w[kWarps], hit_w[kWarps];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  float ce_sum = 0.f, hits = 0.f;
+  for (int b = warp; b < B; b += kWarps) {
+    const float* lr = logits + size_t(b) * C;
+    float mx = -INFINITY;
+    int arg = C;
+    for (int c = lane; c < C; c += 32) {
+      const float v = lr[c];
+      if (v > mx || arg == C) { mx = v; arg = c; }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float om = __shfl_xor_sync(0xffffffffu, mx, o);
+      const int oa = __shfl_xor_sync(0xffffffffu, arg, o);
+      if (om > mx || (om == mx && oa < arg)) { mx = om; arg = oa; }
+    }
+    float s = 0.f;
+    for (int c = lane; c < C; c += 32) s += expf(lr[c] - mx);
+    s = warp_sum(s);
+    const int64_t y = labels[b];
+    const bool valid = y >= 0 && y < C;
+    const float lse = mx + logf(s);
+    ce_sum += valid ? lse - lr[valid ? y : 0] : NAN;
+    hits += (valid && arg == int(y)) ? 1.f : 0.f;
+  }
+  if (lane == 0) {
+    ce_w[warp] = ce_sum;
+    hit_w[warp] = hits;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float a = 0.f, h = 0.f;
+    for (int w = 0; w < kWarps; ++w) {
+      a += ce_w[w];
+      h += hit_w[w];
+    }
+    acc[0] += a;
+    acc[1] += h;
+  }
+}
+
 // dW[c,d] = sum_b dlogits[b,c] * xn[b,d] ; db[c] = sum_b dlogits[b,c]
 __global__ void head_wgrad_kernel(const float* __restrict__ dlogits, const __nv_bfloat16* __restrict__ xn,
                                   float* __restrict__ dW, float* __restrict__ db, int B, int D, int C) {
@@ -314,6 +365,15 @@ int cross_entropy(const float* logits, const int64_t* labels, float* dlogits, fl
                   float loss_scale, cudaStream_t s) {
   APLA_CHECK(B > 0 && C > 0, "cross_entropy: empty");
   ce_kernel<<<B, 256, 0, s>>>(logits, labels, dlogits, loss, C, grad_scale, loss_scale);
+  APLA_CUDA(cudaGetLastError());
+  count_launch();
+  return 0;
+}
+
+int eval_accumulate(const float* logits, const int64_t* labels, int B, int C, float* acc, cudaStream_t s) {
+  APLA_CHECK(B > 0 && C > 0, "apla_eval_accumulate: empty problem B=%d C=%d", B, C);
+  APLA_CHECK(logits && labels && acc, "apla_eval_accumulate: null buffer");
+  eval_acc_kernel<<<1, kEvalThreads, 0, s>>>(logits, labels, B, C, acc);
   APLA_CUDA(cudaGetLastError());
   count_launch();
   return 0;

@@ -6,7 +6,7 @@
 namespace apla {
 
 enum { EPI_BIAS = 0, EPI_BIAS_GELU = 1, EPI_RESID = 2, EPI_GELU_BWD = 3, EPI_F32_T = 4, EPI_DELTA = 5, EPI_BIAS_GELU_D = 6,
-       EPI_MUL_F16 = 7, EPI_RED = 8, EPI_RESID_LN = 9 };
+       EPI_MUL_F16 = 7, EPI_RED = 8, EPI_RESID_LN = 9, EPI_BIAS_GELU_G = 10 };
 
 // gemm.cu
 int gemm_tn(int epi, const void* A, const void* B, int M, int N, int K, int lda, int ldb, void* out, void* out2,
@@ -75,6 +75,7 @@ int assemble_tokens(const void* patch, const float* cls, const float* pos, float
 int head_fwd(const void* xn, const float* W, const float* bias, float* logits, int B, int D, int C, cudaStream_t s);
 int cross_entropy(const float* logits, const int64_t* labels, float* dlogits, float* loss, int B, int C,
                   float grad_scale, float loss_scale, cudaStream_t s);
+int eval_accumulate(const float* logits, const int64_t* labels, int B, int C, float* acc, cudaStream_t s);
 int head_bwd(const float* dlogits, const void* xn, const float* W, float* dW, float* db, void* dxn, int B, int D, int C,
              cudaStream_t s);
 int grad_sumsq(const float* g, int64_t n, float scale, float* out, cudaStream_t s);

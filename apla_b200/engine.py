@@ -14,6 +14,8 @@ Memory layout in HBM (T = B*N tokens, D embed, L blocks), sized for B=64 ViT-B/1
   qkv[l]    bf16 [T, 3D]  ao[l] bf16 [T, D]  lse[l] fp32 [T, H]  hpre[l] fp16 [T, 4D] (gelu' of the fc1 pre-activation)   saved for backward
   ln_out, gelu_out, dx, dxb, dO, dqkv, dsub, delta                                         transients, reused
   params / grads / exp_avg / exp_avg_sq   fp32 arenas [W1 x L | fc.weight | b1 x L | fc.bias]  (one all-reduce)
+  infer_*   evaluation workspace of predict / embed / evaluate (eval_batch_size images, allocated on first use): two fp32
+            [T_eval, D] residual buffers and one block's transients -- no checkpoints, nothing kept for backward
 """
 from __future__ import annotations
 
@@ -51,7 +53,8 @@ def interpolate_pos_table(pos_embed: torch.Tensor, npatch: int) -> torch.Tensor:
 class FineTuneEngine:
     def __init__(self, model: nn.Module, batch_size: int, img_size: int, device="cuda", lr: float = 3e-5,
                  weight_decay: float = 1e-5, clip: float = 1.0, betas=(0.9, 0.999), adam_eps: float = 1e-8,
-                 process_group=None, cls_only_last_block: bool = True, use_graph: bool = True):
+                 process_group=None, cls_only_last_block: bool = True, use_graph: bool = True,
+                 eval_batch_size: Optional[int] = None):
         require_device()
         # Only norm(x)[:, 0] of the last block reaches the head (vit.py:417-419): its projection, LayerNorm 2, MLP and
         # their input gradients run on the CLS rows only.  False = every token (identical results, for A/B checks).
@@ -73,6 +76,12 @@ class FineTuneEngine:
         self._graph_seen: Dict[tuple, int] = {}
         self._keep: List[torch.Tensor] = []          # every device buffer the engine points at
         self._handle = None
+        # predict / embed / evaluate run up to this many images per native call over a workspace of their own, allocated
+        # on first use (about 5 MB per image at ViT-B/14, 518 px, against about 78 MB for the training step)
+        self.eval_batch_size = int(eval_batch_size) if eval_batch_size is not None else int(batch_size)
+        if self.eval_batch_size < 1:
+            raise ValueError("eval_batch_size must be >= 1")
+        self._infer_ws: Optional[Dict[str, torch.Tensor]] = None
         self._build(model, batch_size, img_size)
 
     # ------------------------------------------------------------------------------------------------------------
@@ -609,6 +618,81 @@ class FineTuneEngine:
         st["done"][last].synchronize()
         st["pending"][last] = False
         return float(st["loss_host"][last][0])
+
+    # ---- evaluation (Trainer.evaluate / test, src/defaults/trainer.py:162-345) ----------------------------------------
+    def _infer_workspace(self) -> Dict[str, torch.Tensor]:
+        if self._infer_ws is None:
+            s, cap = self.shape, self.eval_batch_size
+            T, P, D = cap * s["N"], cap * s["P"], s["D"]
+            ws = dict(infer_x=torch.empty(2, T, D, dtype=F32, device=self.device),
+                      infer_ln=torch.empty(T, D, dtype=BF16, device=self.device),
+                      infer_qkv=torch.empty(T, 3 * D, dtype=BF16, device=self.device),
+                      infer_ao=torch.empty(T, D, dtype=BF16, device=self.device),
+                      infer_lse=torch.empty(T, s["H"], dtype=F32, device=self.device),
+                      infer_gelu=torch.empty(T, s["hidden"], dtype=BF16, device=self.device),
+                      infer_patches=torch.empty(P, s["kpad"], dtype=BF16, device=self.device),
+                      infer_pe_out=torch.empty(P, D, dtype=BF16, device=self.device),
+                      infer_cls_ln=torch.empty(cap, D, dtype=BF16, device=self.device))
+            for name, t in ws.items():
+                self._set(name, t)
+            LIB.call("apla_engine_set_option", self._handle, b"infer_batch", cap)
+            self._infer_ws = ws
+        return self._infer_ws
+
+    def _infer(self, images: torch.Tensor, want_emb: bool):
+        """-> (logits fp32 [n, C], bf16 embedding [n, D] or None), chunk by chunk of eval_batch_size images."""
+        img = self.shape["img"]
+        if images.dim() != 4 or tuple(images.shape[1:]) != (3, img, img) or images.shape[0] < 1:
+            raise RuntimeError(f"images must be [n >= 1, 3, {img}, {img}], got {tuple(images.shape)}")
+        if images.dtype != F32:
+            raise RuntimeError("images must be fp32")
+        self._infer_workspace()
+        n = images.shape[0]
+        logits = torch.empty(n, self.shape["C"], dtype=F32, device=self.device)
+        emb = torch.empty(n, self.shape["D"], dtype=BF16, device=self.device) if want_emb else None
+        for i in range(0, n, self.eval_batch_size):
+            chunk = images[i:i + self.eval_batch_size].to(self.device, non_blocking=True).contiguous()
+            LIB.call("apla_engine_infer", self._handle, ptr(chunk), chunk.shape[0], ptr(logits[i:]),
+                     ptr(emb[i:]) if emb is not None else None, stream())
+        return logits, emb
+
+    @torch.no_grad()
+    def predict(self, images: torch.Tensor) -> torch.Tensor:
+        """Classifier.forward (models.py:81-92) with the engine's current weights: fp32 images [n, 3, S, S] (device or
+        host, any n >= 1) -> a new fp32 logits tensor [n, C].  Runs in chunks of `eval_batch_size`; the training
+        buffers, and so the captured step graphs, are left as they are."""
+        return self._infer(images, want_emb=False)[0]
+
+    @torch.no_grad()
+    def embed(self, images: torch.Tensor) -> torch.Tensor:
+        """Classifier.forward(x, return_embedding=True)'s embedding (models.py:88-92), the input of the reference's kNN
+        evaluation (trainer.py:347-455): the final-norm CLS row the head reads, [n, D], as fp32 values of its bf16."""
+        return self._infer(images, want_emb=True)[1].float()
+
+    @torch.no_grad()
+    def evaluate(self, batches) -> Dict[str, float]:
+        """Mean cross-entropy and top-1 accuracy over an iterable of (images, labels) batches on the device or on the host
+        (host batches are copied with non_blocking=True; pinned memory makes that asynchronous).  The sums stay on the
+        device until the end; with a process group they are all-reduced once, so every rank returns the same numbers.
+        -> {"loss": mean CE, "top1": fraction of correct argmax, "n": number of images}."""
+        acc = torch.zeros(2, dtype=F32, device=self.device)
+        n = 0
+        for images, labels in batches:
+            labels = labels.to(self.device, non_blocking=True).contiguous()
+            if labels.dtype != torch.int64 or labels.dim() != 1 or labels.shape[0] != images.shape[0]:
+                raise RuntimeError("labels must be int64 [n] matching the images")
+            logits = self.predict(images)
+            LIB.call("apla_eval_accumulate", ptr(logits), ptr(labels), logits.shape[0], logits.shape[1], ptr(acc), stream())
+            n += int(labels.shape[0])
+        tot = torch.cat([acc.double(), torch.tensor([float(n)], dtype=torch.float64, device=self.device)])
+        if self._dist_on() and self.world > 1:
+            if torch.distributed.get_backend(self.pg) == "gloo":
+                tot = tot.cpu()
+            torch.distributed.all_reduce(tot, group=self.pg)
+        loss_sum, hits, count = tot.tolist()
+        if count == 0:
+            raise ValueError("evaluate() got no batches")
+        return {"loss": loss_sum / count, "top1": hits / count, "n": int(count)}
 
     def grad_norm(self) -> torch.Tensor:
         """sqrt of the sum of squares the last optim_step clipped with (after the 1/world scaling)."""

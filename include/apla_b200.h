@@ -75,6 +75,10 @@ int apla_gemm_bias_gelu_dgelu_fwd(const void* A, int lda, const void* W, int ldw
                                   void* g, int ldo, int M, int N, int K, apla_stream_t stream);
 int apla_gemm_dgrad_mul(const void* dY, int ldy, const void* Wt, int ldwt, const void* mul, void* dH, int ldh, int M,
                         int K_in, int N_out, apla_stream_t stream);
+/* Forward-only fc1 (evaluation, or any forward that autograd will not differentiate): g_bf16 = gelu_erf(A . W^T + bias),
+ * bit-identical to the g output of apla_gemm_bias_gelu_dgelu_fwd; no derivative is written. */
+int apla_gemm_bias_gelu_only_fwd(const void* A, int lda, const void* W, int ldw, const float* bias, void* g, int ldo,
+                                 int M, int N, int K, apla_stream_t stream);
 /* dO_bf16[M,D] = dY_bf16[M,D_out] . Wt^T  and  delta_f32[M, D/64] = rowsum over each 64-wide head of dO * O_bf16:
  * the input gradient of the attention projection (backward of appla_attn.py:64-79) fused with the softmax-backward
  * row term of the attention that produced O (appla_attn.py:58-62); pass the result to apla_attn_bwd with out = NULL. */
@@ -144,6 +148,10 @@ int apla_head_fwd(const void* xn, const float* W, const float* bias, float* logi
 /* *loss += loss_scale * sum_b CE_b ; dlogits = grad_scale * (softmax - onehot)   (wrappers.py:314). */
 int apla_cross_entropy(const float* logits, const int64_t* labels, float* dlogits, float* loss, int B, int C,
                        float grad_scale, float loss_scale, apla_stream_t stream);
+/* Evaluation sums of one batch (Trainer.evaluate, trainer.py:162-245): acc_f32[0] += sum_b CE_b, acc_f32[1] += number of
+ * rows whose argmax (first maximum) equals the label.  One launch, fixed summation order, no host synchronisation; a
+ * label outside [0, C) makes acc[0] NaN. */
+int apla_eval_accumulate(const float* logits, const int64_t* labels, int B, int C, float* acc, apla_stream_t stream);
 /* dW_f32[C,D], db_f32[C] (overwritten) and dxn_bf16[B,D]. */
 int apla_head_bwd(const float* dlogits, const void* xn, const float* W, float* dW, float* db, void* dxn, int B, int D,
                   int C, apla_stream_t stream);
@@ -272,6 +280,12 @@ int apla_block_weights_size(void);
 int apla_block_fwd(const apla_block_weights* w, const float* x_in, float* x_mid, float* x_out, void* ln_tmp, void* qkv,
                    void* ao, float* lse, void* dgelu, void* gelu_tmp, const int32_t* cu_seqlens, int num_seqs,
                    int max_seqlen, int T, apla_stream_t stream);
+/* The same forward keeping nothing for backward (no autograd, evaluation, a frozen teacher): fc1 writes gelu(h) only and
+ * there is no dgelu.  lse_tmp f32[T,H], ln_tmp, qkv, ao and gelu_tmp are scratch.  x_out may alias x_in (x_in is last
+ * read by the projection); x_mid may alias neither. */
+int apla_block_fwd_infer(const apla_block_weights* w, const float* x_in, float* x_mid, float* x_out, void* ln_tmp,
+                         void* qkv, void* ao, float* lse_tmp, void* gelu_tmp, const int32_t* cu_seqlens, int num_seqs,
+                         int max_seqlen, int T, apla_stream_t stream);
 /* dx_out f32[T,D] -> dx_in f32[T,D] (NULL: no input gradient wanted; may alias dx_mid) and dw1 f32[r,D] / db1 f32[r]
  * (NULL: no weight gradient; zeroed here).  dx_mid f32[T,D], dyb bf16[T,D], dh bf16[T,hidden], dln bf16[T,D],
  * dsub bf16[T,r_pad] (compact path), d_ao bf16[T,D], delta f32[T,H], dqkv bf16[T,3D] are scratch.
@@ -295,7 +309,8 @@ apla_engine_t apla_engine_create(int B, int N, int D, int H, int L, int hidden, 
                                  int r, int r_pad, int full_rows, float eps, float scale);
 void apla_engine_destroy(apla_engine_t e);
 int apla_engine_set_ptr(apla_engine_t e, const char* name, int block, void* p);
-/* Options (default in brackets): "cls_only_last_block" [2] -- evaluate the per-token tail of the LAST block (projection,
+/* Options (default in brackets): "infer_batch" [0] -- images per apla_engine_infer call (its workspace capacity);
+ * "cls_only_last_block" [2] -- evaluate the per-token tail of the LAST block (projection,
  * LayerNorm 2, MLP and their input gradients; value >= 1) and its attention (value 2: apla_attn_cls_*) for the CLS
  * rows only, because only norm(x)[:, 0] reaches the head (vit.py:417-419, models.py:87); 0 = every token.  Values 0 and
  * 1 give bit-identical logits / loss; 2 replaces bf16 tensor-core attention of that row by fp32 arithmetic. */
@@ -307,6 +322,14 @@ int64_t apla_engine_arena_decay_size(apla_engine_t e);
 /* logits (+ loss and dlogits when labels != NULL): loss += loss_scale * sum CE, dlogits *= grad_scale. */
 int apla_engine_forward(apla_engine_t e, const float* images, const int64_t* labels, float loss_scale,
                         float grad_scale, apla_stream_t stream);
+/* Evaluation forward: logits_f32[n_img, C] (and, with emb != NULL, the bf16 final-norm CLS rows emb[n_img, D] the head
+ * reads) for 1 <= n_img <= "infer_batch" images with the CURRENT weights (arena + refreshed projection copies).  Runs the
+ * forward's launch sequence with the forward-only fc1 over its own workspace, registered by name (block = -1):
+ * "infer_x" f32[2, cap*N, D], "infer_ln" bf16[cap*N, D], "infer_qkv" bf16[cap*N, 3D], "infer_ao" bf16[cap*N, D],
+ * "infer_lse" f32[cap*N, H], "infer_gelu" bf16[cap*N, hidden], "infer_patches" bf16[cap*P, kpad],
+ * "infer_pe_out" bf16[cap*P, D], "infer_cls_ln" bf16[cap, D].  Reads no buffer of the step but the weights and writes
+ * none: captured step graphs stay valid. */
+int apla_engine_infer(apla_engine_t e, const float* images, int n_img, float* logits, void* emb, apla_stream_t stream);
 /* Backward through blocks block_from, block_from-1, ..., block_to (block_from == L-1 also zeroes the gradient arena
  * and runs the head / final-norm backward first).  Splitting the range lets the host start the data-parallel
  * all-reduce of the upper blocks' gradients while the lower blocks are still running. */
