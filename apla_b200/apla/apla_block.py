@@ -29,6 +29,7 @@ output has the input's dtype.  CUDA (sm_100a) only, no fallback; dropout / drop-
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes
 import os
 import weakref
@@ -37,6 +38,7 @@ from typing import List, Optional, Sequence
 import torch
 import torch.nn as nn
 
+from .. import ops
 from .._lib import LIB, BlockWeights, ptr, require_device, stream
 from .appla_attn import APLA_Attention, _pad64
 
@@ -148,6 +150,9 @@ def _drop_rate(mod) -> float:
 class FusedAplaBlock(nn.Module):
     """Holds the wrapped block's sub-modules under their own names; only `forward` is replaced."""
 
+    # set by `attention_probabilities(model)`: forward(x, return_attention=True) returns the attention probabilities
+    _attention_probs = False
+
     def __init__(self, block: nn.Module):
         super().__init__()
         if not isinstance(block.attn, APLA_Attention):
@@ -252,11 +257,31 @@ class FusedAplaBlock(nn.Module):
                  ptr(ao), ptr(lse), ptr(gelu_tmp), ptr(cu), num_seqs, max_len, T, stream())
         return x_out.view(x.shape).to(x.dtype)
 
+    def _attention(self, x):
+        """The reference Block's `return_attention=True` result (vit.py:282-283): LayerNorm 1, the qkv GEMM, the attention
+        forward for its log-sum-exp, then the fp32 [B,H,N,N] probabilities; the rest of the block is not run."""
+        at = self.attn
+        B, N, D = x.shape
+        ws, ms = at._working_set(x.device), self._mlp_working_set(x.device)
+        x_in = x.detach().reshape(-1, D).to(torch.float32).contiguous()
+        ln = ops.layernorm_fwd(x_in, ms["ln1w"], ms["ln1b"], float(self.norm1.eps))
+        qkv = ops.gemm_bias(ln, ws["wqkv"], ws["bqkv"])
+        _, lse = ops.attn_fwd(qkv, at.num_heads, float(at.scale), B, N)
+        return ops.attn_probs(qkv, lse, at.num_heads, float(at.scale), B, N)
+
     def forward(self, x_or_x_list, return_attention: bool = False, return_intermediate: bool = False):
-        """`[B,N,D]` -> `[B,N,D]` (vit.py:279-288) or list of `[b_i,N_i,D]` -> list (dinov2 block.py:274-288)."""
-        if return_attention or return_intermediate:
-            raise RuntimeError("the fused block never materialises the [B,H,N,N] attention probabilities "
-                               "(vit.py:282-287 visualisation paths): un-fuse the model for them")
+        """`[B,N,D]` -> `[B,N,D]` (vit.py:279-288) or list of `[b_i,N_i,D]` -> list (dinov2 block.py:274-288).
+        Inside `attention_probabilities(model)`, `forward(x, return_attention=True)` on a `[B,N,D]` tensor returns the
+        fp32 [B,H,N,N] attention probabilities of the block (no autograd history), as the reference Block does."""
+        if return_intermediate or (return_attention and not self._attention_probs):
+            raise RuntimeError("the fused block does not materialise the [B,H,N,N] attention probabilities "
+                               "(vit.py:282-287 visualisation paths) unless it runs inside "
+                               "apla_b200.apla.attention_probabilities(model); return_intermediate is not supported")
+        if return_attention:
+            if not isinstance(x_or_x_list, torch.Tensor) or x_or_x_list.dim() != 3:
+                raise RuntimeError("attention probabilities need a dense [B, N, D] tensor, not a list of crops")
+            self._check(x_or_x_list)
+            return self._attention(x_or_x_list)
         if isinstance(x_or_x_list, torch.Tensor):
             self._check(x_or_x_list)
             return self._run_fused(x_or_x_list)
@@ -292,6 +317,27 @@ class PackedCropList(list):
         if len(self) != len(self._views) or any(a is not b for a, b in zip(self, self._views)):
             return None
         return self._packed
+
+
+@contextlib.contextmanager
+def attention_probabilities(model: nn.Module):
+    """Within the block, every `APLA_Attention` of `model` returns `(out, attn)` with `attn` the fp32 [B,H,N,N]
+    attention probabilities (dense inputs; no autograd history), and every `FusedAplaBlock` answers
+    `forward(x, return_attention=True)` with them, as the reference's modules do (appla_attn.py:83, vit.py:282-287).
+    The previous settings are restored on exit, also on an exception and when blocks nest.  Outside it nothing
+    changes: the probabilities are never computed."""
+    mods = [m for m in model.modules() if isinstance(m, (APLA_Attention, FusedAplaBlock))]
+    saved = [m.__dict__.get("_attention_probs") for m in mods]
+    try:
+        for m in mods:
+            m._attention_probs = True
+        yield model
+    finally:
+        for m, v in zip(mods, saved):
+            if v is None:
+                m.__dict__.pop("_attention_probs", None)
+            else:
+                m._attention_probs = v
 
 
 _CU_CACHE = {}

@@ -40,7 +40,7 @@ def _pad64(n: int) -> int:
 
 class _AplaAttentionFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, x, w1, b1, mod, cu_seqlens, seqlens):
+    def forward(ctx, x, w1, b1, mod, cu_seqlens, seqlens, want_attn=False):
         ws = mod._working_set(x.device)
         shape = x.shape
         C = shape[-1]
@@ -53,14 +53,18 @@ class _AplaAttentionFn(torch.autograd.Function):
         qkv = ops.gemm_bias(xb, ws["wqkv"], ws["bqkv"])
         ao, lse = ops.attn_fwd(qkv, mod.num_heads, float(mod.scale), num_seqs, max_len, cu_seqlens=cu_seqlens)
         y = ops.gemm_bias(ao, ws["wproj"], ws["bproj"])
+        if want_attn:                # the probabilities of this very forward, from its qkv and lse (dense input only)
+            attn = ops.attn_probs(qkv, lse, mod.num_heads, float(mod.scale), num_seqs, max_len)
+            ctx.mark_non_differentiable(attn)
         ctx.mod, ctx.ws = mod, ws
         ctx.geom = (num_seqs, max_len, cu_seqlens)
         ctx.x_dtype, ctx.x_shape = x.dtype, shape
         ctx.save_for_backward(qkv, ao, lse)
-        return y.view(shape).to(x.dtype)
+        y = y.view(shape).to(x.dtype)
+        return (y, attn) if want_attn else y
 
     @staticmethod
-    def backward(ctx, dy):
+    def backward(ctx, dy, *_):
         mod, ws = ctx.mod, ctx.ws
         qkv, ao, lse = ctx.saved_tensors
         num_seqs, max_len, cu = ctx.geom
@@ -83,10 +87,13 @@ class _AplaAttentionFn(torch.autograd.Function):
             dqkv = ops.attn_bwd(qkv, None, d_ao, lse, mod.num_heads, float(mod.scale), num_seqs, max_len,
                                 cu_seqlens=cu, delta=delta)
             dx = ops.gemm_dgrad(dqkv, ws["wqkvT"]).view(ctx.x_shape).to(ctx.x_dtype)
-        return dx, dw1, db1, None, None, None
+        return dx, dw1, db1, None, None, None, None
 
 
 class APLA_Attention(nn.Module):
+    # set by `apla_b200.apla.attention_probabilities(model)`: forward then also returns the [B,H,N,N] probabilities
+    _attention_probs = False
+
     def __init__(self, config, dim, indices=None, num_heads=8, qkv_bias=False, qk_scale=None, attn_drop=0.,
                  proj_drop=0.):
         super().__init__()
@@ -181,7 +188,7 @@ class APLA_Attention(nn.Module):
             self._ws_train_key = train_key
         return self._ws
 
-    def _run(self, x, cu_seqlens=None, seqlens=None):
+    def _run(self, x, cu_seqlens=None, seqlens=None, want_attn=False):
         if not x.is_cuda:
             raise RuntimeError("apla_b200.APLA_Attention runs on CUDA (sm_100a) only; there is no CPU fallback")
         require_device()
@@ -189,9 +196,17 @@ class APLA_Attention(nn.Module):
             raise RuntimeError("fused APLA attention supports dropout p=0 only (all shipped reference configs use 0)")
         if self.proj_weight1.device != x.device:
             raise RuntimeError("module parameters and input are on different devices")
-        return _AplaAttentionFn.apply(x, self.proj_weight1, self.proj_bias1, self, cu_seqlens, seqlens)
+        return _AplaAttentionFn.apply(x, self.proj_weight1, self.proj_bias1, self, cu_seqlens, seqlens, want_attn)
 
     def forward(self, x):
         """x [B,N,C] -> (out [B,N,C], attn).  The reference returns the [B,H,N,N] probabilities, which the fused
-        kernel never materialises; `attn` is None (its only consumers are visualisation paths, vit.py:282-287)."""
-        return self._run(x), None
+        kernel does not materialise: `attn` is None (its only consumers are visualisation paths, vit.py:282-287), unless
+        the module is inside `apla_b200.apla.attention_probabilities(...)`.  There `attn` is the fp32 [B,H,N,N] softmax
+        of this call (contiguous, rebuilt by one extra kernel from the forward's own qkv and log-sum-exp) with no
+        autograd history: no gradient flows through it.  `out` and the gradients come from the same launches as without
+        it (the extra kernel only reads qkv and lse)."""
+        if not self._attention_probs:
+            return self._run(x), None
+        if x.dim() != 3:
+            raise RuntimeError(f"attention probabilities need a dense [B, N, C] input, got shape {tuple(x.shape)}")
+        return self._run(x, want_attn=True)

@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(CSRC, "build")
 LIB = os.path.join(HERE, "libapla_b200.so")
-SOURCES = ["common.cu", "gemm.cu", "gemm2.cu", "attention.cu", "attention_tc.cu", "attention_tc_bwd.cu", "attention_fused.cu", "attention_bwd2.cu", "attention_fwd_sr.cu", "attention_cls.cu", "rowwise.cu", "head_optim.cu", "dp_allreduce.cu", "ssl.cu", "engine.cu", "block.cu", "capi.cu"]
+SOURCES = ["common.cu", "gemm.cu", "gemm2.cu", "attention.cu", "attention_tc.cu", "attention_tc_bwd.cu", "attention_fused.cu", "attention_bwd2.cu", "attention_fwd_sr.cu", "attention_cls.cu", "attention_probs.cu", "rowwise.cu", "head_optim.cu", "dp_allreduce.cu", "ssl.cu", "engine.cu", "block.cu", "capi.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "--use_fast_math",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v", "-DNDEBUG"] + os.environ.get("APLA_NVCC_EXTRA", "").split()
 

@@ -124,6 +124,11 @@ int apla_attn_cls_bwd(const void* qkv, const void* out, const void* dout, const 
   return attn_cls_bwd(qkv, out, dout, lse, dqkv, B, N, H, scale, S(stream));
 }
 
+int apla_attn_probs(const void* qkv, const float* lse, float* probs, int B, int N, int H, int q_rows, float scale,
+                    apla_stream_t stream) {
+  return attn_probs(qkv, lse, probs, B, N, H, q_rows, scale, S(stream));
+}
+
 int apla_patchify(const float* images, void* patches, int B, int Simg, int patch, int kpad, apla_stream_t stream) {
   return patchify(images, patches, B, Simg, patch, kpad, S(stream));
 }

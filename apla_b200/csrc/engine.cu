@@ -224,8 +224,10 @@ static int check_infer_ready(Engine* e, int n_img) {
 
 // Classifier.forward (models.py:81-92) for n_img images with the engine's current weights, in the launch sequence of
 // engine_forward (same kernels, same gemm_resid_ln pairing, same CLS-only last block), but over its own workspace and
-// with the forward-only fc1 epilogue: nothing is kept for a backward pass.
-static int engine_infer(Engine* e, const float* images, int n_img, float* logits, void* emb, cudaStream_t s) {
+// with the forward-only fc1 epilogue: nothing is kept for a backward pass.  With cls_probs set it stops after the last
+// block's attention and writes that attention's CLS-query probabilities cls_probs_f32[n_img, H, N] instead of logits.
+static int engine_infer(Engine* e, const float* images, int n_img, float* logits, void* emb, cudaStream_t s,
+                        float* cls_probs = nullptr) {
   if (int rc = check_infer_ready(e, n_img)) return rc;
   const int B = n_img, N = e->N, D = e->D, L = e->L, Hd = e->hidden, T = B * N;
   float* xa = e->get<float>("infer_x");                       // block input, then block output
@@ -259,6 +261,7 @@ static int engine_infer(Engine* e, const float* images, int n_img, float* logits
     } else {
       if (int rc = attn_fwd(qkv, ao, lse, nullptr, B, N, T, e->H, e->scale, s)) return rc;
     }
+    if (cls_probs && l == L - 1) return attn_probs(qkv, lse, cls_probs, B, N, e->H, 1, e->scale, s);
     const int R = cls ? B : T;
     const int sD = cls ? N * D : D, sH = cls ? N * Hd : Hd;
     if (int rc = gemm_resid_ln(ao, b.wproj, R, D, D, sD, D, xb, b.bproj, b.g1, xa, sD, b.ln2w, b.ln2b, ln, sD, e->eps, s))
@@ -508,6 +511,12 @@ int apla_engine_infer(apla_engine_t h, const float* images, int n_img, float* lo
   Engine* e = reinterpret_cast<Engine*>(h);
   APLA_CHECK(e != nullptr && images != nullptr && logits != nullptr, "apla_engine_infer: null handle, images or logits");
   return engine_infer(e, images, n_img, logits, emb, reinterpret_cast<cudaStream_t>(stream));
+}
+int apla_engine_cls_attention(apla_engine_t h, const float* images, int n_img, float* probs, apla_stream_t stream) {
+  Engine* e = reinterpret_cast<Engine*>(h);
+  APLA_CHECK(e != nullptr && images != nullptr && probs != nullptr,
+             "apla_engine_cls_attention: null handle, images or probs");
+  return engine_infer(e, images, n_img, nullptr, nullptr, reinterpret_cast<cudaStream_t>(stream), probs);
 }
 int apla_engine_backward(apla_engine_t h, int block_from, int block_to, apla_stream_t stream) {
   Engine* e = reinterpret_cast<Engine*>(h);

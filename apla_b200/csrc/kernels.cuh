@@ -56,6 +56,10 @@ int attn_cls_fwd(const void* qkv, void* out, float* lse, int B, int N, int H, fl
 int attn_cls_bwd(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv, int B, int N, int H,
                  float scale, cudaStream_t stream);
 
+// attention_probs.cu: probs_f32[B, H, q_rows, N] = exp(scale q k^T - lse) of the first q_rows queries per sequence
+int attn_probs(const void* qkv, const float* lse, float* probs, int B, int N, int H, int q_rows, float scale,
+               cudaStream_t stream);
+
 // rowwise.cu
 int layernorm_fwd(const float* x, int64_t ldx, const float* w, const float* b, void* y, int64_t ldy, int rows, int D,
                   float eps, cudaStream_t stream);

@@ -639,13 +639,16 @@ class FineTuneEngine:
             self._infer_ws = ws
         return self._infer_ws
 
-    def _infer(self, images: torch.Tensor, want_emb: bool):
-        """-> (logits fp32 [n, C], bf16 embedding [n, D] or None), chunk by chunk of eval_batch_size images."""
+    def _check_eval_images(self, images: torch.Tensor):
         img = self.shape["img"]
         if images.dim() != 4 or tuple(images.shape[1:]) != (3, img, img) or images.shape[0] < 1:
             raise RuntimeError(f"images must be [n >= 1, 3, {img}, {img}], got {tuple(images.shape)}")
         if images.dtype != F32:
             raise RuntimeError("images must be fp32")
+
+    def _infer(self, images: torch.Tensor, want_emb: bool):
+        """-> (logits fp32 [n, C], bf16 embedding [n, D] or None), chunk by chunk of eval_batch_size images."""
+        self._check_eval_images(images)
         self._infer_workspace()
         n = images.shape[0]
         logits = torch.empty(n, self.shape["C"], dtype=F32, device=self.device)
@@ -668,6 +671,22 @@ class FineTuneEngine:
         """Classifier.forward(x, return_embedding=True)'s embedding (models.py:88-92), the input of the reference's kNN
         evaluation (trainer.py:347-455): the final-norm CLS row the head reads, [n, D], as fp32 values of its bf16."""
         return self._infer(images, want_emb=True)[1].float()
+
+    @torch.no_grad()
+    def cls_attention(self, images: torch.Tensor) -> torch.Tensor:
+        """The last block's attention of the CLS query over all N tokens, `get_last_selfattention(x)[:, :, 0, :]`
+        (vit.py:439-485), with the engine's current weights: fp32 images [n, 3, S, S] (device or host, any n >= 1) -> a new
+        fp32 tensor [n, H, N] whose rows sum to 1.  Runs like `predict` (chunks of `eval_batch_size` over the same
+        workspace, training buffers and captured graphs untouched) and stops after the last block's attention.  For full
+        [N, N] maps or other blocks, `sync_to_model()` and use `apla_b200.apla.attention_probabilities` on the model."""
+        self._check_eval_images(images)
+        self._infer_workspace()
+        n, s = images.shape[0], self.shape
+        probs = torch.empty(n, s["H"], s["N"], dtype=F32, device=self.device)
+        for i in range(0, n, self.eval_batch_size):
+            chunk = images[i:i + self.eval_batch_size].to(self.device, non_blocking=True).contiguous()
+            LIB.call("apla_engine_cls_attention", self._handle, ptr(chunk), chunk.shape[0], ptr(probs[i:]), stream())
+        return probs
 
     @torch.no_grad()
     def evaluate(self, batches) -> Dict[str, float]:

@@ -271,6 +271,26 @@ def attn_cls_bwd(qkv, out, dout, lse, H: int, scale: float, B: int, N: int, dqkv
     return dqkv
 
 
+def attn_probs(qkv, lse, H: int, scale: float, B: int, N: int, q_rows: Optional[int] = None, out=None):
+    """fp32 [B, H, q_rows, N] attention probabilities of the first q_rows (default N) queries of each of the B dense
+    sequences, from the qkv and lse of the forward (`attn_fwd`, or `attn_cls_fwd` for q_rows = 1)."""
+    require_device()
+    _chk(qkv, BF16, "qkv", 2); _chk(lse, F32, "lse", 2)
+    q_rows = N if q_rows is None else int(q_rows)
+    if qkv.shape != (B * N, 3 * H * 64) or not qkv.is_contiguous():
+        raise RuntimeError(f"qkv must be contiguous [{B * N}, {3 * H * 64}], got {tuple(qkv.shape)}")
+    if lse.shape != (B * N, H) or not lse.is_contiguous():
+        raise RuntimeError(f"lse must be contiguous [{B * N}, {H}], got {tuple(lse.shape)}")
+    if out is None:
+        out = torch.empty(B, H, q_rows, N, device=qkv.device, dtype=F32)
+    else:
+        _chk(out, F32, "out")
+        if out.numel() < B * H * q_rows * N or not out.is_contiguous():
+            raise RuntimeError(f"out must be contiguous with at least {B * H * q_rows * N} elements")
+    LIB.call("apla_attn_probs", ptr(qkv), ptr(lse), ptr(out), B, N, H, q_rows, scale, stream())
+    return out
+
+
 def gemm_bias_ls_accumulate(a, w, bias, gamma, out):
     """out_f32 += gamma * (a @ w^T + bias), in place (TMA reduce-add epilogue)."""
     require_device()

@@ -136,6 +136,13 @@ int apla_attn_cls_fwd(const void* qkv, void* out, float* lse, int B, int N, int 
 int apla_attn_cls_bwd(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv, int B, int N,
                       int H, float scale, apla_stream_t stream);
 
+/* Attention probabilities (the [B,H,N,N] `attn` of appla_attn.py:56-60,83, or its first q_rows query rows):
+ * probs_f32[B, H, q_rows, N] = exp(scale * q k^T - lse) for B dense sequences of N tokens, from the qkv and the lse that
+ * apla_attn_fwd wrote (or, for q_rows = 1, apla_attn_cls_fwd: only the lse of rows b*N is read).  One pass, no softmax
+ * re-normalisation: each row sums to 1 up to rounding.  Refuses NULL pointers, B / N / H < 1 and q_rows outside [1, N]. */
+int apla_attn_probs(const void* qkv, const float* lse, float* probs, int B, int N, int H, int q_rows, float scale,
+                    apla_stream_t stream);
+
 /* --- step ends ------------------------------------------------------------------------------------------ */
 /* patches_bf16[B*P, kpad] from images_f32[B,3,S,S], k = (c, py, px): PatchEmbed conv as a GEMM, vit.py:302-306. */
 int apla_patchify(const float* images, void* patches, int B, int S, int patch, int kpad, apla_stream_t stream);
@@ -330,6 +337,12 @@ int apla_engine_forward(apla_engine_t e, const float* images, const int64_t* lab
  * "infer_pe_out" bf16[cap*P, D], "infer_cls_ln" bf16[cap, D].  Reads no buffer of the step but the weights and writes
  * none: captured step graphs stay valid. */
 int apla_engine_infer(apla_engine_t e, const float* images, int n_img, float* logits, void* emb, apla_stream_t stream);
+/* CLS attention map of the last block (vit.py get_last_selfattention(x)[:, :, 0, :]): probs_f32[n_img, H, N] for
+ * 1 <= n_img <= "infer_batch" images with the CURRENT weights.  The launch sequence of apla_engine_infer up to and
+ * including the last block's attention (any "cls_only_last_block" mode), then apla_attn_probs with q_rows = 1; that
+ * block's tail, the final norm and the head are not run.  Same workspace and the same argument checks as
+ * apla_engine_infer. */
+int apla_engine_cls_attention(apla_engine_t e, const float* images, int n_img, float* probs, apla_stream_t stream);
 /* Backward through blocks block_from, block_from-1, ..., block_to (block_from == L-1 also zeroes the gradient arena
  * and runs the head / final-norm backward first).  Splitting the range lets the host start the data-parallel
  * all-reduce of the upper blocks' gradients while the lower blocks are still running. */
