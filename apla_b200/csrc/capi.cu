@@ -144,6 +144,10 @@ int apla_cross_entropy(const float* logits, const int64_t* labels, float* dlogit
                        float grad_scale, float loss_scale, apla_stream_t stream) {
   return cross_entropy(logits, labels, dlogits, loss, B, C, grad_scale, loss_scale, S(stream));
 }
+int apla_cross_entropy_soft(const float* logits, const float* targets, float* dlogits, float* loss, int B, int C,
+                            float grad_scale, float loss_scale, apla_stream_t stream) {
+  return cross_entropy_soft(logits, targets, dlogits, loss, B, C, grad_scale, loss_scale, S(stream));
+}
 int apla_eval_accumulate(const float* logits, const int64_t* labels, int B, int C, float* acc, apla_stream_t stream) {
   return eval_accumulate(logits, labels, B, C, acc, S(stream));
 }

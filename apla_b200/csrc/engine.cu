@@ -52,6 +52,9 @@ struct Engine {
   int side_wgrad = 0;
   // evaluation forward (apla_engine_infer): images per call at most, set by option "infer_batch"; 0 = no workspace
   int infer_cap = 0;
+  // images of the last training forward (apla_engine_forward_n; B for apla_engine_forward): the backward consumes that
+  // forward's saved activations, so it runs over the same n_cur * N rows
+  int n_cur = 0;
   cudaStream_t side = nullptr;
   std::vector<cudaEvent_t> ev_fork, ev_done;
   ~Engine() {
@@ -133,11 +136,17 @@ static Arena arena_of(const Engine* e) {
   return a;
 }
 
-static int engine_forward(Engine* e, const float* images, const int64_t* labels, float loss_scale, float grad_scale,
-                          cudaStream_t s) {
+// The step's forward over the first n images of its buffers (n = B: the full batch).  Every launch covers n*N token rows
+// or n CLS rows, so rows beyond them -- stale from an earlier, larger batch -- are never read; only the xs checkpoints
+// keep their capacity stride TD.
+static int engine_forward(Engine* e, const float* images, int n, const int64_t* labels, const float* targets,
+                          float loss_scale, float grad_scale, cudaStream_t s) {
+  APLA_CHECK(n >= 1 && n <= e->B, "apla_engine_forward_n: n_img=%d outside [1, %d]", n, e->B);
+  APLA_CHECK(!(labels && targets), "apla_engine_forward_n: labels and targets are both set");
   if (int rc = check_ready(e)) return rc;
-  const int T = e->T(), D = e->D, B = e->B, N = e->N, L = e->L, Hd = e->hidden;
-  const size_t TD = size_t(T) * D;
+  const int D = e->D, B = n, N = e->N, L = e->L, Hd = e->hidden, T = B * N;
+  const size_t TD = size_t(e->T()) * D;
+  e->n_cur = n;
   float* xs = e->get<float>("xs");
   void* ln_out = e->get<void>("ln_out");
   void* gelu_out = e->get<void>("gelu_out");
@@ -198,11 +207,17 @@ static int engine_forward(Engine* e, const float* images, const int64_t* labels,
     return rc;
   if (int rc = head_fwd(e->get<void>("cls_ln"), params + ar.fcw, params + ar.fcb, e->get<float>("logits"), B, D, e->C, s))
     return rc;
-  if (labels) {
+  if (labels || targets) {
     APLA_CUDA(cudaMemsetAsync(e->get<float>("loss"), 0, sizeof(float), s));
-    if (int rc = cross_entropy(e->get<float>("logits"), labels, e->get<float>("dlogits"), e->get<float>("loss"), B, e->C,
-                               grad_scale, loss_scale, s))
-      return rc;
+    if (labels) {
+      if (int rc = cross_entropy(e->get<float>("logits"), labels, e->get<float>("dlogits"), e->get<float>("loss"), B, e->C,
+                                 grad_scale, loss_scale, s))
+        return rc;
+    } else {
+      if (int rc = cross_entropy_soft(e->get<float>("logits"), targets, e->get<float>("dlogits"), e->get<float>("loss"), B,
+                                      e->C, grad_scale, loss_scale, s))
+        return rc;
+    }
   }
   return 0;
 }
@@ -283,15 +298,16 @@ static int engine_infer(Engine* e, const float* images, int n_img, float* logits
 
 static int engine_backward(Engine* e, int l_from, int l_to, cudaStream_t s) {
   if (int rc = check_ready(e)) return rc;
-  const int T = e->T(), D = e->D, B = e->B, N = e->N, L = e->L, Hd = e->hidden, r = e->r;
-  const size_t TD = size_t(T) * D;
+  // rows of the last forward (n_cur images); the xs checkpoints and the two dsub slots keep their capacity strides
+  const int D = e->D, B = e->n_cur, N = e->N, L = e->L, Hd = e->hidden, r = e->r, T = B * N;
+  const size_t TD = size_t(e->T()) * D, Tn_D = size_t(T) * D;
   float* xs = e->get<float>("xs");
   void* dln = e->get<void>("ln_out");      // reused: gradient w.r.t. a LayerNorm output
   void* dH = e->get<void>("gelu_out");     // reused: gradient w.r.t. the fc1 pre-activation
   float* dx = e->get<float>("dx");
   void* dxb = e->get<void>("dxb");
   char* dsub0 = e->full_rows ? nullptr : e->get<char>("dsub");
-  const size_t dsub_bytes = size_t(T) * e->r_pad * 2;
+  const size_t dsub_slot = size_t(e->T()) * e->r_pad * 2, dsub_bytes = size_t(T) * e->r_pad * 2;
   const bool side = e->side_wgrad >= 2 || (e->side_wgrad >= 1 && e->full_rows);
   if (side) {
     if (int rc = e->side_ready()) return rc;
@@ -310,8 +326,8 @@ static int engine_backward(Engine* e, int l_from, int l_to, cudaStream_t s) {
                         e->get<void>("dcls"), B, D, e->C, s))
     return rc;
   // final norm backward: only CLS rows carry gradient; everything else in dx / dxb is zero
-  APLA_CUDA(cudaMemsetAsync(dx, 0, TD * sizeof(float), s));
-  APLA_CUDA(cudaMemsetAsync(dxb, 0, TD * 2, s));
+  APLA_CUDA(cudaMemsetAsync(dx, 0, Tn_D * sizeof(float), s));
+  APLA_CUDA(cudaMemsetAsync(dxb, 0, Tn_D * 2, s));
   if (int rc = layernorm_bwd(e->get<void>("dcls"), D, xs + size_t(2 * L) * TD, int64_t(N) * D, e->get<float>("lnfw"),
                              nullptr, 0, dx, int64_t(N) * D, dxb, int64_t(N) * D, e->blk[L - 1].g2, nullptr, 0, nullptr, 0,
                              0, B, D, e->eps, s))
@@ -334,7 +350,7 @@ static int engine_backward(Engine* e, int l_from, int l_to, cudaStream_t s) {
       return rc;
     // dsub alternates between two slots when the weight gradient runs beside the main chain: block l's LayerNorm-2
     // backward may only overwrite the slot after block l+2's weight gradient has read it
-    void* dsub = dsub0 ? dsub0 + ((side && (l & 1)) ? dsub_bytes : 0) : nullptr;
+    void* dsub = dsub0 ? dsub0 + ((side && (l & 1)) ? dsub_slot : 0) : nullptr;
     if (side && dsub && l + 2 <= l_from) APLA_CUDA(cudaStreamWaitEvent(s, e->ev_done[l + 2], 0));
     if (cls && dsub) APLA_CUDA(cudaMemsetAsync(dsub, 0, dsub_bytes, s));
     // dx_mid = dx_out + LN2'(dln); dxb = bf16(gamma1 * dx_mid); dsub = its APLA columns
@@ -437,6 +453,7 @@ apla_engine_t apla_engine_create(int B, int N, int D, int H, int L, int hidden, 
   Engine* e = new Engine();
   e->B = B; e->N = N; e->D = D; e->H = H; e->L = L; e->hidden = hidden; e->C = C; e->P = N - 1; e->patch = patch;
   e->img = img; e->kpad = kpad; e->r = r; e->r_pad = r_pad; e->full_rows = full_rows; e->eps = eps; e->scale = scale;
+  e->n_cur = B;
   e->blk.resize(L);
   return e;
 }
@@ -505,7 +522,13 @@ int apla_engine_forward(apla_engine_t h, const float* images, const int64_t* lab
                         apla_stream_t stream) {
   Engine* e = reinterpret_cast<Engine*>(h);
   APLA_CHECK(e != nullptr && images != nullptr, "apla_engine_forward: null handle or images");
-  return engine_forward(e, images, labels, loss_scale, grad_scale, reinterpret_cast<cudaStream_t>(stream));
+  return engine_forward(e, images, e->B, labels, nullptr, loss_scale, grad_scale, reinterpret_cast<cudaStream_t>(stream));
+}
+int apla_engine_forward_n(apla_engine_t h, const float* images, int n_img, const int64_t* labels, const float* targets,
+                          float loss_scale, float grad_scale, apla_stream_t stream) {
+  Engine* e = reinterpret_cast<Engine*>(h);
+  APLA_CHECK(e != nullptr && images != nullptr, "apla_engine_forward_n: null handle or images");
+  return engine_forward(e, images, n_img, labels, targets, loss_scale, grad_scale, reinterpret_cast<cudaStream_t>(stream));
 }
 int apla_engine_infer(apla_engine_t h, const float* images, int n_img, float* logits, void* emb, apla_stream_t stream) {
   Engine* e = reinterpret_cast<Engine*>(h);

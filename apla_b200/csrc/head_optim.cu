@@ -63,6 +63,56 @@ __global__ void ce_kernel(const float* __restrict__ logits, const int64_t* __res
   if (threadIdx.x == 0) atomicAdd(loss, (lse - lr[y]) * loss_scale);
 }
 
+// Probability targets t[b, :] (F.cross_entropy(z, t) with fp32 [B, C] targets: mixup / cutmix / label smoothing), neither
+// normalised nor validated, as torch does neither:  loss_b = tsum lse - tz with tsum = sum_c t_c, tz = sum_c t_c z_c;
+// dlogits = (tsum softmax - t) * grad_scale.  The max / exponential-sum passes and the block reductions are ce_kernel's,
+// with tsum and tz reduced beside the sum: for a one-hot row tsum == 1.0f and every zero term adds exactly, so lse, the
+// row loss and (1.0f * p - t) * grad_scale are ce_kernel's bit for bit.
+__global__ void ce_soft_kernel(const float* __restrict__ logits, const float* __restrict__ targets,
+                               float* __restrict__ dlogits, float* __restrict__ loss, int C, float grad_scale,
+                               float loss_scale) {
+  const int b = blockIdx.x;
+  const float* lr = logits + size_t(b) * C;
+  const float* tr = targets + size_t(b) * C;
+  __shared__ float red[32], red_t[32], red_tz[32];
+  float mx = -INFINITY;
+  for (int c = threadIdx.x; c < C; c += blockDim.x) mx = fmaxf(mx, lr[c]);
+  mx = warp_max(mx);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = mx;
+  __syncthreads();
+  mx = red[0];
+  for (int i = 1; i < (blockDim.x >> 5); ++i) mx = fmaxf(mx, red[i]);
+  __syncthreads();
+  float s = 0.f, ts = 0.f, tz = 0.f;
+  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+    const float z = lr[c], t = tr[c];
+    s += expf(z - mx);
+    ts += t;
+    tz += t * z;
+  }
+  s = warp_sum(s);
+  ts = warp_sum(ts);
+  tz = warp_sum(tz);
+  if ((threadIdx.x & 31) == 0) {
+    red[threadIdx.x >> 5] = s;
+    red_t[threadIdx.x >> 5] = ts;
+    red_tz[threadIdx.x >> 5] = tz;
+  }
+  __syncthreads();
+  s = 0.f;
+  ts = 0.f;
+  tz = 0.f;
+  for (int i = 0; i < (blockDim.x >> 5); ++i) {
+    s += red[i];
+    ts += red_t[i];
+    tz += red_tz[i];
+  }
+  const float lse = mx + logf(s);
+  for (int c = threadIdx.x; c < C; c += blockDim.x)
+    dlogits[size_t(b) * C + c] = (ts * expf(lr[c] - lse) - tr[c]) * grad_scale;
+  if (threadIdx.x == 0) atomicAdd(loss, (ts * lse - tz) * loss_scale);
+}
+
 // Evaluation sums over one batch, one CTA: acc[0] += sum_b CE_b (the row softmax of ce_kernel, one warp per row),
 // acc[1] += #{b : argmax_c logits[b,c] == labels[b]} with the first maximum winning, as torch.argmax picks it.  Each warp
 // walks its rows in order and the warps' partial sums are added in warp order: the result does not depend on timing.
@@ -365,6 +415,16 @@ int cross_entropy(const float* logits, const int64_t* labels, float* dlogits, fl
                   float loss_scale, cudaStream_t s) {
   APLA_CHECK(B > 0 && C > 0, "cross_entropy: empty");
   ce_kernel<<<B, 256, 0, s>>>(logits, labels, dlogits, loss, C, grad_scale, loss_scale);
+  APLA_CUDA(cudaGetLastError());
+  count_launch();
+  return 0;
+}
+
+int cross_entropy_soft(const float* logits, const float* targets, float* dlogits, float* loss, int B, int C,
+                       float grad_scale, float loss_scale, cudaStream_t s) {
+  APLA_CHECK(B > 0 && C > 0, "cross_entropy_soft: empty problem B=%d C=%d", B, C);
+  APLA_CHECK(logits && targets && dlogits && loss, "cross_entropy_soft: null buffer");
+  ce_soft_kernel<<<B, 256, 0, s>>>(logits, targets, dlogits, loss, C, grad_scale, loss_scale);
   APLA_CUDA(cudaGetLastError());
   count_launch();
   return 0;

@@ -79,6 +79,8 @@ int assemble_tokens(const void* patch, const float* cls, const float* pos, float
 int head_fwd(const void* xn, const float* W, const float* bias, float* logits, int B, int D, int C, cudaStream_t s);
 int cross_entropy(const float* logits, const int64_t* labels, float* dlogits, float* loss, int B, int C,
                   float grad_scale, float loss_scale, cudaStream_t s);
+int cross_entropy_soft(const float* logits, const float* targets, float* dlogits, float* loss, int B, int C,
+                       float grad_scale, float loss_scale, cudaStream_t s);
 int eval_accumulate(const float* logits, const int64_t* labels, int B, int C, float* acc, cudaStream_t s);
 int head_bwd(const float* dlogits, const void* xn, const float* W, float* dW, float* db, void* dxn, int B, int D, int C,
              cudaStream_t s);

@@ -76,6 +76,7 @@ class FineTuneEngine:
         self._graph_seen: Dict[tuple, int] = {}
         self._keep: List[torch.Tensor] = []          # every device buffer the engine points at
         self._handle = None
+        self.buffers: Dict[tuple, Optional[torch.Tensor]] = {}
         # predict / embed / evaluate run up to this many images per native call over a workspace of their own, allocated
         # on first use (about 5 MB per image at ViT-B/14, 518 px, against about 78 MB for the training step)
         self.eval_batch_size = int(eval_batch_size) if eval_batch_size is not None else int(batch_size)
@@ -100,6 +101,7 @@ class FineTuneEngine:
 
     def _set(self, name: str, t: Optional[torch.Tensor], block: int = -1):
         LIB.call("apla_engine_set_ptr", self._handle, name.encode(), block, ptr(t))
+        self.buffers[(name, block)] = t       # what the native engine points at, by name (block -1: global)
 
     def _build(self, model, B, img):
         bb = model.backbone
@@ -395,21 +397,54 @@ class FineTuneEngine:
         return ckpt
 
     # ------------------------------------------------------------------------------------------------------------
-    def _check_inputs(self, images, labels):
-        B = self.shape["B"]
-        if images.shape != self.images_dev.shape or images.dtype != F32 or not images.is_cuda:
-            raise RuntimeError(f"images must be a CUDA fp32 tensor of shape {tuple(self.images_dev.shape)}")
-        if labels is not None and (labels.dtype != torch.int64 or labels.shape != (B,) or not labels.is_cuda):
-            raise RuntimeError("labels must be a CUDA int64 tensor of shape [B]")
+    def _check_inputs(self, images, labels, on_device: bool = True) -> int:
+        """-> n, the number of images of a training batch: fp32 images [n, 3, S, S] with 1 <= n <= batch_size, and labels
+        either int64 class indices [n] or fp32 class probabilities [n, C] (what F.cross_entropy takes: a DataLoader's
+        partial last batch, AdvancedAugCollate's mixup / cutmix / label-smoothed targets)."""
+        B, img, C = self.shape["B"], self.shape["img"], self.shape["C"]
+        where = "CUDA " if on_device else ""
+        if (images.dim() != 4 or tuple(images.shape[1:]) != (3, img, img) or images.dtype != F32
+                or (on_device and not images.is_cuda)):
+            raise RuntimeError(f"images must be a {where}fp32 tensor of shape [n, 3, {img}, {img}] with 1 <= n <= {B}, "
+                               f"got {images.dtype} {tuple(images.shape)}")
+        n = int(images.shape[0])
+        if not 1 <= n <= B:
+            raise RuntimeError(f"a step takes 1 to batch_size={B} images, got {n}")
+        if labels is None:
+            return n
+        if on_device and not labels.is_cuda:
+            raise RuntimeError("labels must be a CUDA tensor")
+        if labels.dtype == torch.int64:
+            if tuple(labels.shape) != (n,):
+                raise RuntimeError(f"int64 labels must have shape [{n}] (one class index per image), got {tuple(labels.shape)}")
+        elif labels.dtype == F32:
+            if tuple(labels.shape) != (n, C):
+                raise RuntimeError(f"fp32 targets must have shape [{n}, {C}] (class probabilities per image), got "
+                                   f"{tuple(labels.shape)}")
+        else:
+            raise RuntimeError(f"labels must be int64 [n] class indices or fp32 [n, C] class probabilities, got {labels.dtype}")
+        return n
+
+    def _launch_forward(self, images: torch.Tensor, labels: Optional[torch.Tensor], n: int):
+        # CrossEntropyLoss(mean) over the local batch of n images (wrappers.py:314); DDP later averages over ranks.  The
+        # full hard-label batch keeps its original entry point; a partial batch or probability targets take the n-row one.
+        inv = 1.0 / n
+        if n == self.shape["B"] and (labels is None or labels.dtype == torch.int64):
+            LIB.call("apla_engine_forward", self._handle, ptr(images), ptr(labels), inv, inv, stream())
+            return
+        soft = labels is not None and labels.dtype == F32
+        LIB.call("apla_engine_forward_n", self._handle, ptr(images), n, None if soft else ptr(labels),
+                 ptr(labels) if soft else None, inv, inv, stream())
 
     def forward(self, images: torch.Tensor, labels: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """images fp32 [B,3,S,S] on the engine's device -> logits fp32 [B,C] (and loss/dlogits when labels given)."""
-        B = self.shape["B"]
-        self._check_inputs(images, labels)
+        """images fp32 [n,3,S,S] (1 <= n <= B) on the engine's device -> logits fp32 [n,C], a view of the first n rows of
+        `self.logits` (and loss / dlogits when labels are given: int64 [n] class indices or fp32 [n, C] probabilities).
+        The next backward() runs over the same n images."""
+        n = self._check_inputs(images, labels)
         images = images.contiguous()
-        # CrossEntropyLoss(mean) over the local batch (wrappers.py:314); DDP later averages gradients over ranks
-        LIB.call("apla_engine_forward", self._handle, ptr(images), ptr(labels), 1.0 / B, 1.0 / B, stream())
-        return self.logits
+        labels = labels.contiguous() if labels is not None else None
+        self._launch_forward(images, labels, n)
+        return self.logits if n == self.shape["B"] else self.logits[:n]
 
     def backward(self):
         L = self.shape["L"]
@@ -468,7 +503,8 @@ class FineTuneEngine:
                  self.betas[0], self.betas[1], self.adam_eps, self.step_count, stream())
 
     def step(self, images: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:
-        """One Trainer.global_step on device-resident inputs; returns the (device) loss scalar."""
+        """One Trainer.global_step on device-resident inputs -- fp32 images [n, 3, S, S] with 1 <= n <= batch_size, int64
+        labels [n] or fp32 targets [n, C] -- with the mean loss over the n images; returns the (device) loss scalar."""
         if not self.use_graph:
             self.forward(images, labels)
             self.backward()
@@ -478,7 +514,11 @@ class FineTuneEngine:
         # sequence, nothing executes during capture) and replayed from then on
         if not images.is_contiguous():
             images = images.contiguous()      # (a fresh buffer every call: stays on the eager path)
-        key = (images.data_ptr(), labels.data_ptr(), tuple(images.shape))
+        if not labels.is_contiguous():
+            labels = labels.contiguous()
+        # the row count (images.shape) and the label kind (dtype / shape) are baked into a captured step: a partial batch
+        # gets a graph of its own, captured on its second sighting like any buffer pair
+        key = (images.data_ptr(), labels.data_ptr(), tuple(images.shape), labels.dtype, tuple(labels.shape))
         g = self._graphs.get(key)
         if g is None:
             seen = self._graph_seen.get(key, 0)
@@ -488,12 +528,9 @@ class FineTuneEngine:
                 self.backward()
                 self.optim_step()
                 return self.loss
-            self._check_inputs(images, labels)
-            if not images.is_contiguous():
-                raise RuntimeError("images must be contiguous")
+            n = self._check_inputs(images, labels)
             torch.cuda.current_stream().synchronize()
             L = self.shape["L"]
-            inv_b = 1.0 / self.shape["B"]
 
             def capture(fn):
                 gr = torch.cuda.CUDAGraph()
@@ -511,7 +548,7 @@ class FineTuneEngine:
 
             if self.world == 1:
                 def whole():
-                    LIB.call("apla_engine_forward", self._handle, ptr(images), ptr(labels), inv_b, inv_b, stream())
+                    self._launch_forward(images, labels, n)
                     LIB.call("apla_engine_backward", self._handle, L - 1, 0, stream())
                     optim()
                 g = (capture(whole),)
@@ -519,7 +556,7 @@ class FineTuneEngine:
                 # data parallel with the native all-reduce: ONE graph; the early slice's reduction is forked onto the
                 # side stream inside the capture and joins before the optimiser
                 def whole_dp():
-                    LIB.call("apla_engine_forward", self._handle, ptr(images), ptr(labels), inv_b, inv_b, stream())
+                    self._launch_forward(images, labels, n)
                     self.backward()
                     optim()
                 g = (capture(whole_dp),)
@@ -528,7 +565,7 @@ class FineTuneEngine:
                 half = ArenaLayout(L=L, r=self.shape["r"], D=self.shape["D"], C=self.shape["C"]).split_block()
 
                 def upper():
-                    LIB.call("apla_engine_forward", self._handle, ptr(images), ptr(labels), inv_b, inv_b, stream())
+                    self._launch_forward(images, labels, n)
                     LIB.call("apla_engine_backward", self._handle, L - 1, half, stream())
 
                 def lower():
@@ -568,7 +605,12 @@ class FineTuneEngine:
         of step k-1) and the loss comes back through a pinned buffer.  With `lag=True` (default) the call returns the
         loss of the PREVIOUS step (None on the first call) so that the host never waits for the step it just enqueued
         -- the same one-step-late logging the reference does every `log_every` (src/defaults/trainer.py:145-151);
-        `lag=False` synchronises and returns this step's loss.  `drain()` returns the last pending loss."""
+        `lag=False` synchronises and returns this step's loss.  `drain()` returns the last pending loss.
+
+        A batch may hold 1 <= n <= batch_size images (a loader's partial last batch) and int64 [n] labels or fp32 [n, C]
+        targets: it is copied into the first n rows of the slot, and the first soft batch allocates a pair of fp32 [B, C]
+        target slots."""
+        n = self._check_inputs(images_pinned, labels_pinned, on_device=False)
         if not hasattr(self, "_e2e"):
             B, img = self.shape["B"], self.shape["img"]
             self._e2e = dict(
@@ -583,14 +625,20 @@ class FineTuneEngine:
         slot = st["slot"]
         st["slot"] = slot ^ 1
         cur = torch.cuda.current_stream()
+        if labels_pinned.dtype == F32 and "tgt" not in st:
+            # allocated on the compute stream that reads them, like the other slots
+            B, C = self.shape["B"], self.shape["C"]
+            st["tgt"] = [self._new(B, C, dtype=F32), self._new(B, C, dtype=F32)]
+        img_dev = st["img"][slot][:n]
+        lab_dev = (st["tgt"] if labels_pinned.dtype == F32 else st["lab"])[slot][:n]
         with torch.cuda.stream(st["copy_stream"]):
             if st["pending"][slot]:
                 st["copy_stream"].wait_event(st["done"][slot])      # the step that last read this slot has finished
-            st["img"][slot].copy_(images_pinned, non_blocking=True)
-            st["lab"][slot].copy_(labels_pinned, non_blocking=True)
+            img_dev.copy_(images_pinned, non_blocking=True)
+            lab_dev.copy_(labels_pinned, non_blocking=True)
             st["copied"][slot].record()
         cur.wait_event(st["copied"][slot])
-        self.step(st["img"][slot], st["lab"][slot])
+        self.step(img_dev, lab_dev)
         st["loss_host"][slot].copy_(self.loss, non_blocking=True)
         st["done"][slot].record(cur)
         st["pending"][slot] = True

@@ -155,6 +155,13 @@ int apla_head_fwd(const void* xn, const float* W, const float* bias, float* logi
 /* *loss += loss_scale * sum_b CE_b ; dlogits = grad_scale * (softmax - onehot)   (wrappers.py:314). */
 int apla_cross_entropy(const float* logits, const int64_t* labels, float* dlogits, float* loss, int B, int C,
                        float grad_scale, float loss_scale, apla_stream_t stream);
+/* Probability targets (nn.CrossEntropyLoss with fp32 [B, C] targets, wrappers.py:314, as timm Mixup / CutMix with label
+ * smoothing yields them, src/utils/_utils.py:424): with tsum_b = sum_c t[b,c] and tz_b = sum_c t[b,c] z[b,c],
+ * *loss += loss_scale * sum_b (tsum_b lse_b - tz_b) ; dlogits = grad_scale * (tsum_b softmax - t).  Targets are neither
+ * normalised nor validated (torch does neither).  For one-hot rows dlogits equals apla_cross_entropy's bit for bit.
+ * Refuses NULL pointers and B or C < 1. */
+int apla_cross_entropy_soft(const float* logits, const float* targets, float* dlogits, float* loss, int B, int C,
+                            float grad_scale, float loss_scale, apla_stream_t stream);
 /* Evaluation sums of one batch (Trainer.evaluate, trainer.py:162-245): acc_f32[0] += sum_b CE_b, acc_f32[1] += number of
  * rows whose argmax (first maximum) equals the label.  One launch, fixed summation order, no host synchronisation; a
  * label outside [0, C) makes acc[0] NaN. */
@@ -329,6 +336,14 @@ int64_t apla_engine_arena_decay_size(apla_engine_t e);
 /* logits (+ loss and dlogits when labels != NULL): loss += loss_scale * sum CE, dlogits *= grad_scale. */
 int apla_engine_forward(apla_engine_t e, const float* images, const int64_t* labels, float loss_scale,
                         float grad_scale, apla_stream_t stream);
+/* The same forward over the first 1 <= n_img <= B images of the step's buffers (the partial last batch of an epoch), with
+ * hard labels int64[n_img] or probability targets f32[n_img, C] (apla_cross_entropy_soft), at most one of the two; with
+ * neither, logits only.  Every GEMM, attention, LayerNorm and the head run over n_img*N rows (n_img CLS rows); the xs
+ * checkpoints keep their capacity stride B*N*D and rows beyond n_img*N of any buffer are neither read nor written.  The
+ * engine records n_img: the next apla_engine_backward runs over the same rows.  apla_engine_forward(...) is
+ * apla_engine_forward_n(e, images, B, labels, NULL, ...). */
+int apla_engine_forward_n(apla_engine_t e, const float* images, int n_img, const int64_t* labels, const float* targets,
+                          float loss_scale, float grad_scale, apla_stream_t stream);
 /* Evaluation forward: logits_f32[n_img, C] (and, with emb != NULL, the bf16 final-norm CLS rows emb[n_img, D] the head
  * reads) for 1 <= n_img <= "infer_batch" images with the CURRENT weights (arena + refreshed projection copies).  Runs the
  * forward's launch sequence with the forward-only fc1 over its own workspace, registered by name (block = -1):
@@ -345,7 +360,8 @@ int apla_engine_infer(apla_engine_t e, const float* images, int n_img, float* lo
 int apla_engine_cls_attention(apla_engine_t e, const float* images, int n_img, float* probs, apla_stream_t stream);
 /* Backward through blocks block_from, block_from-1, ..., block_to (block_from == L-1 also zeroes the gradient arena
  * and runs the head / final-norm backward first).  Splitting the range lets the host start the data-parallel
- * all-reduce of the upper blocks' gradients while the lower blocks are still running. */
+ * all-reduce of the upper blocks' gradients while the lower blocks are still running.  It runs over the n_img images of
+ * the last apla_engine_forward / apla_engine_forward_n, whose saved activations it consumes. */
 int apla_engine_backward(apla_engine_t e, int block_from, int block_to, apla_stream_t stream);
 /* clip + AdamW over the arena, then refresh of the dense bf16 projection copies */
 int apla_engine_optim(apla_engine_t e, float gscale, float max_norm, float lr, float wd, float beta1, float beta2,
