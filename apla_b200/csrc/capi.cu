@@ -151,6 +151,14 @@ int apla_cross_entropy_soft(const float* logits, const float* targets, float* dl
 int apla_eval_accumulate(const float* logits, const int64_t* labels, int B, int C, float* acc, apla_stream_t stream) {
   return eval_accumulate(logits, labels, B, C, acc, S(stream));
 }
+int apla_bce_with_logits(const float* logits, const float* targets, float* dlogits, float* loss, int B, int C,
+                         float grad_scale, float loss_scale, apla_stream_t stream) {
+  return bce_with_logits(logits, targets, dlogits, loss, B, C, grad_scale, loss_scale, S(stream));
+}
+int apla_eval_accumulate_bce(const float* logits, const float* targets, int B, int C, double* acc,
+                             apla_stream_t stream) {
+  return eval_accumulate_bce(logits, targets, B, C, acc, S(stream));
+}
 int apla_head_bwd(const float* dlogits, const void* xn, const float* W, float* dW, float* db, void* dxn, int B, int D,
                   int C, apla_stream_t stream) {
   return head_bwd(dlogits, xn, W, dW, db, dxn, B, D, C, S(stream));

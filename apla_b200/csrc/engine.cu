@@ -55,6 +55,9 @@ struct Engine {
   // images of the last training forward (apla_engine_forward_n; B for apla_engine_forward): the backward consumes that
   // forward's saved activations, so it runs over the same n_cur * N rows
   int n_cur = 0;
+  // training loss, option "criterion": 0 = cross-entropy (int64 labels or fp32 class probabilities), 1 = BCE-with-logits
+  // (fp32 multi-label targets only)
+  int criterion = 0;
   cudaStream_t side = nullptr;
   std::vector<cudaEvent_t> ev_fork, ev_done;
   ~Engine() {
@@ -143,6 +146,8 @@ static int engine_forward(Engine* e, const float* images, int n, const int64_t* 
                           float loss_scale, float grad_scale, cudaStream_t s) {
   APLA_CHECK(n >= 1 && n <= e->B, "apla_engine_forward_n: n_img=%d outside [1, %d]", n, e->B);
   APLA_CHECK(!(labels && targets), "apla_engine_forward_n: labels and targets are both set");
+  APLA_CHECK(!(labels && e->criterion == 1),
+             "apla_engine_forward: criterion 1 (BCE-with-logits) takes fp32 targets [n_img, C], not int64 labels");
   if (int rc = check_ready(e)) return rc;
   const int D = e->D, B = n, N = e->N, L = e->L, Hd = e->hidden, T = B * N;
   const size_t TD = size_t(e->T()) * D;
@@ -212,6 +217,10 @@ static int engine_forward(Engine* e, const float* images, int n, const int64_t* 
     if (labels) {
       if (int rc = cross_entropy(e->get<float>("logits"), labels, e->get<float>("dlogits"), e->get<float>("loss"), B, e->C,
                                  grad_scale, loss_scale, s))
+        return rc;
+    } else if (e->criterion == 1) {
+      if (int rc = bce_with_logits(e->get<float>("logits"), targets, e->get<float>("dlogits"), e->get<float>("loss"), B,
+                                   e->C, grad_scale, loss_scale, s))
         return rc;
     } else {
       if (int rc = cross_entropy_soft(e->get<float>("logits"), targets, e->get<float>("dlogits"), e->get<float>("loss"), B,
@@ -503,6 +512,12 @@ int apla_engine_set_option(apla_engine_t h, const char* name, int value) {
   }
   if (std::string(name) == "side_wgrad") {   // 0 = off, 1 = on for partial_size == dim, 2 = on, "dsub" holds two slots
     e->side_wgrad = value < 0 ? 0 : (value > 2 ? 2 : value);
+    return 0;
+  }
+  if (std::string(name) == "criterion") {   // 0 = cross-entropy, 1 = BCE-with-logits
+    APLA_CHECK(value == 0 || value == 1,
+               "apla_engine_set_option: criterion=%d is neither 0 (cross-entropy) nor 1 (BCE-with-logits)", value);
+    e->criterion = value;
     return 0;
   }
   set_error("apla_engine_set_option: unknown option '%s'", name);

@@ -113,6 +113,42 @@ __global__ void ce_soft_kernel(const float* __restrict__ logits, const float* __
   if (threadIdx.x == 0) atomicAdd(loss, (ts * lse - tz) * loss_scale);
 }
 
+// BCEWithLogitsLoss (pos_weight 1) of one element in fp32, finite for every finite z: with e = exp(-|z|) <= 1,
+// l = max(z, 0) - z t + log1p(e) and sigma(z) = 1 / (1 + e) for z >= 0, e / (1 + e) otherwise.
+__device__ __forceinline__ float bce_term(float z, float t, float& sig) {
+  const float e = expf(-fabsf(z));
+  const float inv = 1.f / (1.f + e);
+  sig = z >= 0.f ? inv : e * inv;
+  return fmaxf(z, 0.f) - z * t + log1pf(e);
+}
+
+// Multi-label targets t[b, :] (nn.BCEWithLogitsLoss, wrappers.py:310-320), neither clamped nor checked, as torch does
+// neither: per row, loss += loss_scale * sum_c l(z, t); dlogits = (sigma(z) - t) * grad_scale.  One CTA per row with the
+// block reduction of ce_kernel, one atomicAdd per row.
+__global__ void bce_kernel(const float* __restrict__ logits, const float* __restrict__ targets,
+                           float* __restrict__ dlogits, float* __restrict__ loss, int C, float grad_scale,
+                           float loss_scale) {
+  const int b = blockIdx.x;
+  const float* lr = logits + size_t(b) * C;
+  const float* tr = targets + size_t(b) * C;
+  __shared__ float red[32];
+  float s = 0.f;
+  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+    const float t = tr[c];
+    float sig;
+    s += bce_term(lr[c], t, sig);
+    dlogits[size_t(b) * C + c] = (sig - t) * grad_scale;
+  }
+  s = warp_sum(s);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    s = 0.f;
+    for (int i = 0; i < (blockDim.x >> 5); ++i) s += red[i];
+    atomicAdd(loss, s * loss_scale);
+  }
+}
+
 // Evaluation sums over one batch, one CTA: acc[0] += sum_b CE_b (the row softmax of ce_kernel, one warp per row),
 // acc[1] += #{b : argmax_c logits[b,c] == labels[b]} with the first maximum winning, as torch.argmax picks it.  Each warp
 // walks its rows in order and the warps' partial sums are added in warp order: the result does not depend on timing.
@@ -157,6 +193,49 @@ __global__ void __launch_bounds__(kEvalThreads) eval_acc_kernel(const float* __r
     float a = 0.f, h = 0.f;
     for (int w = 0; w < kWarps; ++w) {
       a += ce_w[w];
+      h += hit_w[w];
+    }
+    acc[0] += a;
+    acc[1] += h;
+  }
+}
+
+__device__ __forceinline__ double warp_sum_d(double v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+
+// Multi-label evaluation sums over one batch of n = B*C elements, one CTA: acc[0] += sum l (bce_term),
+// acc[1] += #{(b, c) : (z > 0) == (t >= 0.5)}.  The accumulator is double: a validation set's element count passes 2^24,
+// beyond which an fp32 counter stops counting.  Each thread walks its elements in order and sums in double, the warps
+// reduce in a fixed shuffle pattern and thread 0 adds the warps in warp order: the result does not depend on timing.
+__global__ void __launch_bounds__(kEvalThreads) eval_acc_bce_kernel(const float* __restrict__ logits,
+                                                                   const float* __restrict__ targets, int64_t n,
+                                                                   double* __restrict__ acc) {
+  constexpr int kWarps = kEvalThreads / 32;
+  __shared__ double l_w[kWarps], hit_w[kWarps];
+  double l_sum = 0.0;
+  int64_t hits = 0;
+  for (int64_t i = threadIdx.x; i < n; i += kEvalThreads) {
+    const float z = logits[i], t = targets[i];
+    float sig;
+    l_sum += double(bce_term(z, t, sig));
+    hits += (z > 0.f) == (t >= 0.5f);
+  }
+  l_sum = warp_sum_d(l_sum);
+  double h = warp_sum_d(double(hits));
+  const int warp = threadIdx.x >> 5;
+  if ((threadIdx.x & 31) == 0) {
+    l_w[warp] = l_sum;
+    hit_w[warp] = h;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double a = 0.0;
+    h = 0.0;
+    for (int w = 0; w < kWarps; ++w) {
+      a += l_w[w];
       h += hit_w[w];
     }
     acc[0] += a;
@@ -425,6 +504,25 @@ int cross_entropy_soft(const float* logits, const float* targets, float* dlogits
   APLA_CHECK(B > 0 && C > 0, "cross_entropy_soft: empty problem B=%d C=%d", B, C);
   APLA_CHECK(logits && targets && dlogits && loss, "cross_entropy_soft: null buffer");
   ce_soft_kernel<<<B, 256, 0, s>>>(logits, targets, dlogits, loss, C, grad_scale, loss_scale);
+  APLA_CUDA(cudaGetLastError());
+  count_launch();
+  return 0;
+}
+
+int bce_with_logits(const float* logits, const float* targets, float* dlogits, float* loss, int B, int C,
+                    float grad_scale, float loss_scale, cudaStream_t s) {
+  APLA_CHECK(B > 0 && C > 0, "bce_with_logits: empty problem B=%d C=%d", B, C);
+  APLA_CHECK(logits && targets && dlogits && loss, "bce_with_logits: null buffer");
+  bce_kernel<<<B, 256, 0, s>>>(logits, targets, dlogits, loss, C, grad_scale, loss_scale);
+  APLA_CUDA(cudaGetLastError());
+  count_launch();
+  return 0;
+}
+
+int eval_accumulate_bce(const float* logits, const float* targets, int B, int C, double* acc, cudaStream_t s) {
+  APLA_CHECK(B > 0 && C > 0, "apla_eval_accumulate_bce: empty problem B=%d C=%d", B, C);
+  APLA_CHECK(logits && targets && acc, "apla_eval_accumulate_bce: null buffer");
+  eval_acc_bce_kernel<<<1, kEvalThreads, 0, s>>>(logits, targets, int64_t(B) * C, acc);
   APLA_CUDA(cudaGetLastError());
   count_launch();
   return 0;

@@ -82,6 +82,9 @@ int cross_entropy(const float* logits, const int64_t* labels, float* dlogits, fl
 int cross_entropy_soft(const float* logits, const float* targets, float* dlogits, float* loss, int B, int C,
                        float grad_scale, float loss_scale, cudaStream_t s);
 int eval_accumulate(const float* logits, const int64_t* labels, int B, int C, float* acc, cudaStream_t s);
+int bce_with_logits(const float* logits, const float* targets, float* dlogits, float* loss, int B, int C,
+                    float grad_scale, float loss_scale, cudaStream_t s);
+int eval_accumulate_bce(const float* logits, const float* targets, int B, int C, double* acc, cudaStream_t s);
 int head_bwd(const float* dlogits, const void* xn, const float* W, float* dW, float* db, void* dxn, int B, int D, int C,
              cudaStream_t s);
 int grad_sumsq(const float* g, int64_t n, float scale, float* out, cudaStream_t s);

@@ -2,8 +2,9 @@
 
 Takes a classifier built the reference way (`Classifier`: backbone ViT with APLA attention + `fc` head,
 src/defaults/models.py:24-92; here usually `hostvit.HostClassifier`), lays its tensors out for the B200 and runs
-`Trainer.global_step` (src/defaults/trainer.py:106-138) -- forward, CrossEntropy, backward restricted to the APLA
-rows and the head, data-parallel gradient mean, clip_grad_norm_(1.0), AdamW -- as native kernel launches.
+`Trainer.global_step` (src/defaults/trainer.py:106-138) -- forward, the criterion (CrossEntropy, or BCE-with-logits for
+multi-label tasks), backward restricted to the APLA rows and the head, data-parallel gradient mean,
+clip_grad_norm_(1.0), AdamW -- as native kernel launches.
 
 PyTorch's role here is plumbing only: device allocation (torch tensors own every buffer), the one-time conversion
 of frozen fp32 weights into bf16 [out,in] / [in,out] copies, stream handles and torch.distributed/NCCL for the
@@ -36,6 +37,33 @@ def _pad64(n: int) -> int:
     return (n + 63) // 64 * 64
 
 
+def criterion_code(criterion) -> int:
+    """The engine's "criterion" option for the loss a reference trainer built (`DefaultWrapper`, wrappers.py:310-320):
+    None or a default nn.CrossEntropyLoss -> 0, an nn.BCEWithLogitsLoss with reduction="mean" and neither weight nor
+    pos_weight -> 1.  Anything else is refused with a ValueError, so that a step never trains another objective."""
+    supported = ("supported: None or nn.CrossEntropyLoss() (multi-class), nn.BCEWithLogitsLoss() (multi-label), both "
+                 "with default arguments")
+    if criterion is None:
+        return 0
+    if type(criterion) is nn.CrossEntropyLoss:
+        if criterion.label_smoothing > 0:
+            raise ValueError(f"CrossEntropyLoss(label_smoothing={criterion.label_smoothing}) is not supported: pass "
+                             "smoothed fp32 [n, C] targets to step() instead (what timm's Mixup / label smoothing yields); "
+                             + supported)
+        if criterion.reduction != "mean" or criterion.weight is not None or criterion.ignore_index != -100:
+            raise ValueError(f"CrossEntropyLoss(reduction={criterion.reduction!r}, weight="
+                             f"{'set' if criterion.weight is not None else None}, ignore_index={criterion.ignore_index}) "
+                             "is not supported; " + supported)
+        return 0
+    if type(criterion) is nn.BCEWithLogitsLoss:
+        if criterion.reduction != "mean" or criterion.weight is not None or criterion.pos_weight is not None:
+            raise ValueError(f"BCEWithLogitsLoss(reduction={criterion.reduction!r}, weight="
+                             f"{'set' if criterion.weight is not None else None}, pos_weight="
+                             f"{'set' if criterion.pos_weight is not None else None}) is not supported; " + supported)
+        return 1
+    raise ValueError(f"criterion {type(criterion).__name__} is not supported; " + supported)
+
+
 def interpolate_pos_table(pos_embed: torch.Tensor, npatch: int) -> torch.Tensor:
     """Bicubic resize of a [1, 1+n0, D] position table to an npatch grid (vit.py:421-437); done ONCE at engine
     construction because pos_embed is frozen (the reference recomputes it every forward, SURVEY.md K21)."""
@@ -54,7 +82,9 @@ class FineTuneEngine:
     def __init__(self, model: nn.Module, batch_size: int, img_size: int, device="cuda", lr: float = 3e-5,
                  weight_decay: float = 1e-5, clip: float = 1.0, betas=(0.9, 0.999), adam_eps: float = 1e-8,
                  process_group=None, cls_only_last_block: bool = True, use_graph: bool = True,
-                 eval_batch_size: Optional[int] = None):
+                 eval_batch_size: Optional[int] = None, criterion=None):
+        # the trainer's loss (`criterion=self.criterion`): 0 = cross-entropy, 1 = BCE-with-logits (multi-label)
+        self.criterion = criterion_code(criterion)
         require_device()
         # Only norm(x)[:, 0] of the last block reaches the head (vit.py:417-419): its projection, LayerNorm 2, MLP and
         # their input gradients run on the CLS rows only.  False = every token (identical results, for A/B checks).
@@ -130,6 +160,7 @@ class FineTuneEngine:
         if not self._handle:
             raise RuntimeError("apla_engine_create failed: " + LIB.last_error())
         LIB.call("apla_engine_set_option", self._handle, b"cls_only_last_block", int(self.cls_only_last_block))
+        LIB.call("apla_engine_set_option", self._handle, b"criterion", self.criterion)
         # measured: no gain on C2 (7.94 vs 7.98 ms), +0.4 % on C3 -- the step runs into the power cap, not into idle SMs;
         # kept as an option (APLA_SIDE_WGRAD=1), off by default
         self.side_wgrad = os.environ.get("APLA_SIDE_WGRAD", "0") != "0"
@@ -400,7 +431,8 @@ class FineTuneEngine:
     def _check_inputs(self, images, labels, on_device: bool = True) -> int:
         """-> n, the number of images of a training batch: fp32 images [n, 3, S, S] with 1 <= n <= batch_size, and labels
         either int64 class indices [n] or fp32 class probabilities [n, C] (what F.cross_entropy takes: a DataLoader's
-        partial last batch, AdvancedAugCollate's mixup / cutmix / label-smoothed targets)."""
+        partial last batch, AdvancedAugCollate's mixup / cutmix / label-smoothed targets).  A BCE-with-logits engine takes
+        fp32 multi-label targets [n, C] only."""
         B, img, C = self.shape["B"], self.shape["img"], self.shape["C"]
         where = "CUDA " if on_device else ""
         if (images.dim() != 4 or tuple(images.shape[1:]) != (3, img, img) or images.dtype != F32
@@ -414,6 +446,11 @@ class FineTuneEngine:
             return n
         if on_device and not labels.is_cuda:
             raise RuntimeError("labels must be a CUDA tensor")
+        if self.criterion == 1:
+            if labels.dtype != F32 or tuple(labels.shape) != (n, C):
+                raise RuntimeError(f"a BCE-with-logits engine takes fp32 multi-label targets of shape [{n}, {C}], got "
+                                   f"{labels.dtype} {tuple(labels.shape)}")
+            return n
         if labels.dtype == torch.int64:
             if tuple(labels.shape) != (n,):
                 raise RuntimeError(f"int64 labels must have shape [{n}] (one class index per image), got {tuple(labels.shape)}")
@@ -426,9 +463,10 @@ class FineTuneEngine:
         return n
 
     def _launch_forward(self, images: torch.Tensor, labels: Optional[torch.Tensor], n: int):
-        # CrossEntropyLoss(mean) over the local batch of n images (wrappers.py:314); DDP later averages over ranks.  The
-        # full hard-label batch keeps its original entry point; a partial batch or probability targets take the n-row one.
-        inv = 1.0 / n
+        # CrossEntropyLoss(mean) over the local batch of n images (wrappers.py:314), BCEWithLogitsLoss(mean) over its n*C
+        # elements; DDP later averages over ranks.  The full hard-label batch keeps its original entry point; a partial
+        # batch or fp32 targets take the n-row one.
+        inv = 1.0 / n if self.criterion == 0 else 1.0 / (n * self.shape["C"])
         if n == self.shape["B"] and (labels is None or labels.dtype == torch.int64):
             LIB.call("apla_engine_forward", self._handle, ptr(images), ptr(labels), inv, inv, stream())
             return
@@ -438,7 +476,8 @@ class FineTuneEngine:
 
     def forward(self, images: torch.Tensor, labels: Optional[torch.Tensor] = None) -> torch.Tensor:
         """images fp32 [n,3,S,S] (1 <= n <= B) on the engine's device -> logits fp32 [n,C], a view of the first n rows of
-        `self.logits` (and loss / dlogits when labels are given: int64 [n] class indices or fp32 [n, C] probabilities).
+        `self.logits` (and loss / dlogits when labels are given: int64 [n] class indices or fp32 [n, C] probabilities;
+        on a BCE-with-logits engine fp32 [n, C] multi-label targets, with the mean over the n*C elements).
         The next backward() runs over the same n images."""
         n = self._check_inputs(images, labels)
         images = images.contiguous()
@@ -504,7 +543,8 @@ class FineTuneEngine:
 
     def step(self, images: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:
         """One Trainer.global_step on device-resident inputs -- fp32 images [n, 3, S, S] with 1 <= n <= batch_size, int64
-        labels [n] or fp32 targets [n, C] -- with the mean loss over the n images; returns the (device) loss scalar."""
+        labels [n] or fp32 targets [n, C] -- with the mean loss over the n images; returns the (device) loss scalar.  On a
+        BCE-with-logits engine the labels are fp32 multi-label targets [n, C] and the loss is the mean over n*C elements."""
         if not self.use_graph:
             self.forward(images, labels)
             self.backward()
@@ -608,8 +648,8 @@ class FineTuneEngine:
         `lag=False` synchronises and returns this step's loss.  `drain()` returns the last pending loss.
 
         A batch may hold 1 <= n <= batch_size images (a loader's partial last batch) and int64 [n] labels or fp32 [n, C]
-        targets: it is copied into the first n rows of the slot, and the first soft batch allocates a pair of fp32 [B, C]
-        target slots."""
+        targets (on a BCE-with-logits engine: fp32 [n, C] multi-label targets only): it is copied into the first n rows of
+        the slot, and the first fp32-target batch allocates a pair of fp32 [B, C] target slots."""
         n = self._check_inputs(images_pinned, labels_pinned, on_device=False)
         if not hasattr(self, "_e2e"):
             B, img = self.shape["B"], self.shape["img"]
@@ -741,15 +781,26 @@ class FineTuneEngine:
         """Mean cross-entropy and top-1 accuracy over an iterable of (images, labels) batches on the device or on the host
         (host batches are copied with non_blocking=True; pinned memory makes that asynchronous).  The sums stay on the
         device until the end; with a process group they are all-reduced once, so every rank returns the same numbers.
-        -> {"loss": mean CE, "top1": fraction of correct argmax, "n": number of images}."""
-        acc = torch.zeros(2, dtype=F32, device=self.device)
+        -> {"loss": mean CE, "top1": fraction of correct argmax, "n": number of images}.
+
+        On a BCE-with-logits engine the labels are fp32 multi-label targets [n, C], summed in double on the device
+        -> {"loss": mean BCE over the n*C elements, "label_acc": fraction of elements with (logit > 0) == (target >= 0.5),
+        "n": number of images}.  For ranking metrics (ROC-AUC, mAP) take `predict`'s logits."""
+        bce = self.criterion == 1
+        C = self.shape["C"]
+        acc = torch.zeros(2, dtype=torch.float64 if bce else F32, device=self.device)
         n = 0
         for images, labels in batches:
             labels = labels.to(self.device, non_blocking=True).contiguous()
-            if labels.dtype != torch.int64 or labels.dim() != 1 or labels.shape[0] != images.shape[0]:
+            if bce:
+                if labels.dtype != F32 or tuple(labels.shape) != (images.shape[0], C):
+                    raise RuntimeError(f"targets must be fp32 [n, {C}] matching the images, got {labels.dtype} "
+                                       f"{tuple(labels.shape)}")
+            elif labels.dtype != torch.int64 or labels.dim() != 1 or labels.shape[0] != images.shape[0]:
                 raise RuntimeError("labels must be int64 [n] matching the images")
             logits = self.predict(images)
-            LIB.call("apla_eval_accumulate", ptr(logits), ptr(labels), logits.shape[0], logits.shape[1], ptr(acc), stream())
+            LIB.call("apla_eval_accumulate_bce" if bce else "apla_eval_accumulate", ptr(logits), ptr(labels),
+                     logits.shape[0], logits.shape[1], ptr(acc), stream())
             n += int(labels.shape[0])
         tot = torch.cat([acc.double(), torch.tensor([float(n)], dtype=torch.float64, device=self.device)])
         if self._dist_on() and self.world > 1:
@@ -759,6 +810,8 @@ class FineTuneEngine:
         loss_sum, hits, count = tot.tolist()
         if count == 0:
             raise ValueError("evaluate() got no batches")
+        if bce:
+            return {"loss": loss_sum / (count * C), "label_acc": hits / (count * C), "n": int(count)}
         return {"loss": loss_sum / count, "top1": hits / count, "n": int(count)}
 
     def grad_norm(self) -> torch.Tensor:

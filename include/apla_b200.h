@@ -166,6 +166,16 @@ int apla_cross_entropy_soft(const float* logits, const float* targets, float* dl
  * rows whose argmax (first maximum) equals the label.  One launch, fixed summation order, no host synchronisation; a
  * label outside [0, C) makes acc[0] NaN. */
 int apla_eval_accumulate(const float* logits, const int64_t* labels, int B, int C, float* acc, apla_stream_t stream);
+/* Multi-label targets (nn.BCEWithLogitsLoss, wrappers.py:310-320, without weight or pos_weight): per element
+ * l = max(z, 0) - z t + log1p(exp(-|z|)) in fp32, finite for every finite z;  *loss += loss_scale * sum_{b,c} l (one
+ * atomicAdd per row) ; dlogits = grad_scale * (sigmoid(z) - t).  Targets f32[B, C] are neither clamped nor checked (torch
+ * does neither).  BCEWithLogitsLoss's mean is loss_scale = grad_scale = 1 / (B C).  Refuses NULL pointers and B or C < 1. */
+int apla_bce_with_logits(const float* logits, const float* targets, float* dlogits, float* loss, int B, int C,
+                         float grad_scale, float loss_scale, apla_stream_t stream);
+/* Multi-label evaluation sums of one batch: acc_f64[0] += sum_{b,c} l (as apla_bce_with_logits), acc_f64[1] += number of
+ * elements with (z > 0) == (t >= 0.5).  double, because element counts of a validation set pass 2^24.  One launch, fixed
+ * summation order, no host synchronisation.  Refuses NULL pointers and B or C < 1. */
+int apla_eval_accumulate_bce(const float* logits, const float* targets, int B, int C, double* acc, apla_stream_t stream);
 /* dW_f32[C,D], db_f32[C] (overwritten) and dxn_bf16[B,D]. */
 int apla_head_bwd(const float* dlogits, const void* xn, const float* W, float* dW, float* db, void* dxn, int B, int D,
                   int C, apla_stream_t stream);
@@ -327,7 +337,10 @@ int apla_engine_set_ptr(apla_engine_t e, const char* name, int block, void* p);
  * "cls_only_last_block" [2] -- evaluate the per-token tail of the LAST block (projection,
  * LayerNorm 2, MLP and their input gradients; value >= 1) and its attention (value 2: apla_attn_cls_*) for the CLS
  * rows only, because only norm(x)[:, 0] reaches the head (vit.py:417-419, models.py:87); 0 = every token.  Values 0 and
- * 1 give bit-identical logits / loss; 2 replaces bf16 tensor-core attention of that row by fp32 arithmetic. */
+ * 1 give bit-identical logits / loss; 2 replaces bf16 tensor-core attention of that row by fp32 arithmetic;
+ * "criterion" [0] -- the training loss: 0 = cross-entropy (nn.CrossEntropyLoss), 1 = BCE-with-logits
+ * (nn.BCEWithLogitsLoss, multi-label: apla_engine_forward_n reads `targets` as f32[n_img, C] BCE targets and refuses
+ * int64 labels, as apla_engine_forward does); any other value is refused. */
 int apla_engine_set_option(apla_engine_t e, const char* name, int value);
 /* Trainable arena layout (fp32): [proj_weight1 x L | fc.weight | proj_bias1 x L | fc.bias]; the first
  * apla_engine_arena_decay_size() elements are weight-decayed (src/defaults/wrappers.py:205-221). */
@@ -341,7 +354,9 @@ int apla_engine_forward(apla_engine_t e, const float* images, const int64_t* lab
  * neither, logits only.  Every GEMM, attention, LayerNorm and the head run over n_img*N rows (n_img CLS rows); the xs
  * checkpoints keep their capacity stride B*N*D and rows beyond n_img*N of any buffer are neither read nor written.  The
  * engine records n_img: the next apla_engine_backward runs over the same rows.  apla_engine_forward(...) is
- * apla_engine_forward_n(e, images, B, labels, NULL, ...). */
+ * apla_engine_forward_n(e, images, B, labels, NULL, ...).  Under option "criterion" = 1 the loss is BCE-with-logits:
+ * `targets` are f32[n_img, C] multi-label targets (apla_bce_with_logits) and int64 `labels` are refused before any launch;
+ * the backward consumes dlogits whichever criterion produced them. */
 int apla_engine_forward_n(apla_engine_t e, const float* images, int n_img, const int64_t* labels, const float* targets,
                           float loss_scale, float grad_scale, apla_stream_t stream);
 /* Evaluation forward: logits_f32[n_img, C] (and, with emb != NULL, the bf16 final-norm CLS rows emb[n_img, D] the head
