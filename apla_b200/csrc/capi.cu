@@ -36,6 +36,18 @@ int apla_gemm_bias_ls_residual_fwd(const void* A, int lda, const void* W, int ld
                                    apla_stream_t stream) {
   return gemm_tn(EPI_RESID, A, W, M, N, K, lda, ldw, out, nullptr, bias, gamma, resid, ldo, S(stream), 0);
 }
+int apla_gemm_bias_ls_residual_scaled_fwd(const void* A, int lda, const void* W, int ldw, const float* bias,
+                                          const float* gamma, const float* resid, const float* row_scale,
+                                          int rows_per_scale, float* out, int ldo, int M, int N, int K,
+                                          apla_stream_t stream) {
+  if (!A || !W || !resid || !row_scale || !out) {
+    set_error("apla_gemm_bias_ls_residual_scaled_fwd: null A, W, resid, row_scale or out");
+    return 1;
+  }
+  APLA_CHECK(M > 0 && N > 0 && K > 0, "apla_gemm_bias_ls_residual_scaled_fwd: empty problem %dx%dx%d", M, N, K);
+  APLA_CHECK(rows_per_scale >= 1, "apla_gemm_bias_ls_residual_scaled_fwd: rows_per_scale=%d must be >= 1", rows_per_scale);
+  return gemm_resid_scaled(A, W, M, N, K, lda, ldw, out, bias, gamma, resid, ldo, row_scale, rows_per_scale, S(stream));
+}
 int apla_gemm_bias_ls_residual_ln_fwd(const void* A, int lda, const void* W, int ldw, const float* bias,
                                       const float* gamma, const float* resid, float* out, int ldo, const float* ln_w,
                                       const float* ln_b, void* ln_out, int ld_ln, float eps, int M, int N, int K,
@@ -94,6 +106,20 @@ int apla_layernorm_bwd(const void* dy, int64_t ld_dy, const float* x, int64_t ld
                        apla_stream_t stream) {
   return layernorm_bwd(dy, ld_dy, x, ldx, w, dres, ld_dres, dx, ld_dx, dxb, ld_dxb, gamma, sub, ld_sub, idx, r, r_pad,
                        rows, D, eps, S(stream));
+}
+int apla_layernorm_bwd_scaled(const void* dy, int64_t ld_dy, const float* x, int64_t ldx, const float* w,
+                              const float* dres, int64_t ld_dres, float* dx, int64_t ld_dx, void* dxb, int64_t ld_dxb,
+                              const float* gamma, void* sub, int64_t ld_sub, const int32_t* idx, int r, int r_pad,
+                              const float* row_scale, int rows_per_scale, int rows, int D, float eps,
+                              apla_stream_t stream) {
+  if (!dy || !x || !w || !dx || !dxb || !row_scale) {
+    set_error("apla_layernorm_bwd_scaled: null dy, x, w, dx, dxb or row_scale");
+    return 1;
+  }
+  APLA_CHECK(rows > 0 && D > 0, "apla_layernorm_bwd_scaled: empty problem rows=%d D=%d", rows, D);
+  APLA_CHECK(rows_per_scale >= 1, "apla_layernorm_bwd_scaled: rows_per_scale=%d must be >= 1", rows_per_scale);
+  return layernorm_bwd(dy, ld_dy, x, ldx, w, dres, ld_dres, dx, ld_dx, dxb, ld_dxb, gamma, sub, ld_sub, idx, r, r_pad,
+                       rows, D, eps, S(stream), row_scale, rows_per_scale);
 }
 int apla_gather_cols(const void* dy, int64_t ld, void* sub, int64_t ld_sub, const int32_t* idx, int r, int r_pad,
                      int rows, apla_stream_t stream) {

@@ -100,8 +100,18 @@ static const char* kGlobalNames[] = {
 };
 
 // optional global buffers (not checked by check_ready): "hyper" = float[3] {lr, 1 - beta1^t, sqrt(1 - beta2^t)} read by
-// the AdamW kernel instead of its launch arguments, so that a captured step can be replayed with new values
-static const char* kOptionalNames[] = {"hyper"};
+// the AdamW kernel instead of its launch arguments, so that a captured step can be replayed with new values;
+// "drop_path" = float[L, 2, B] stochastic-depth scales s[l, branch, image] in {0, 1/keep} (vit.py drop_path), written by
+// the host before every training forward (see drop_path_scale)
+static const char* kOptionalNames[] = {"hyper", "drop_path"};
+
+// Scales of block l's branch (0 = attention, 1 = MLP) for the images of a step, or NULL without drop path.  The branch
+// output of image b is multiplied by s[l, branch, b] in the forward (EPI_RESID_SCALED), and so is the bf16 gradient the
+// branch reads in the backward (the row-scaled LayerNorm backward); the fp32 residual gradient passes unscaled.
+static const float* drop_path_scale(Engine* e, int l, int branch) {
+  const float* s = e->get<float>("drop_path");
+  return s ? s + size_t(2 * l + branch) * e->B : nullptr;
+}
 
 // evaluation workspace (apla_engine_infer), sized for infer_cap images of N tokens; none of it is used by the step.
 // "infer_x" holds two fp32 [cap*N, D] residual buffers: the block input (overwritten by the block output) and the stream
@@ -187,9 +197,10 @@ static int engine_forward(Engine* e, const float* images, int n, const int64_t* 
     }
     const int R = cls ? B : T;
     const int sD = cls ? N * D : D, sH = cls ? N * Hd : Hd;
+    const int rps = cls ? 1 : N;   // rows per image: the scale of drop path is one per image
     // projection (+bias, LayerScale, residual) and LayerNorm 2 in one launch
     if (int rc = gemm_resid_ln(b.ao, b.wproj, R, D, D, sD, D, x_mid, b.bproj, b.g1, x_in, sD, b.ln2w, b.ln2b, ln_out, sD,
-                               e->eps, s))
+                               e->eps, s, -1, drop_path_scale(e, l, 0), rps))
       return rc;
     if (int rc = gemm_tn(EPI_BIAS_GELU_D, ln_out, b.wfc1, R, Hd, D, sD, D, b.hpre, gelu_out, b.bfc1, nullptr, nullptr, sH, s, 0))
       return rc;
@@ -197,7 +208,10 @@ static int engine_forward(Engine* e, const float* images, int n, const int64_t* 
       // fc2 (+bias, LayerScale, residual) and the NEXT block's LayerNorm 1 in one launch
       const BlockPtrs& nb = e->blk[l + 1];
       if (int rc = gemm_resid_ln(gelu_out, b.wfc2, R, D, Hd, sH, Hd, x_out, b.bfc2, b.g2, x_mid, sD, nb.ln1w, nb.ln1b, ln_out,
-                                 sD, e->eps, s))
+                                 sD, e->eps, s, -1, drop_path_scale(e, l, 1), rps))
+        return rc;
+    } else if (const float* dp = drop_path_scale(e, l, 1)) {
+      if (int rc = gemm_resid_scaled(gelu_out, b.wfc2, R, D, Hd, sH, Hd, x_out, b.bfc2, b.g2, x_mid, sD, dp, rps, s))
         return rc;
     } else {
       if (int rc = gemm_tn(EPI_RESID, gelu_out, b.wfc2, R, D, Hd, sH, Hd, x_out, nullptr, b.bfc2, b.g2, x_mid, sD, s, 0))
@@ -339,7 +353,7 @@ static int engine_backward(Engine* e, int l_from, int l_to, cudaStream_t s) {
   APLA_CUDA(cudaMemsetAsync(dxb, 0, Tn_D * 2, s));
   if (int rc = layernorm_bwd(e->get<void>("dcls"), D, xs + size_t(2 * L) * TD, int64_t(N) * D, e->get<float>("lnfw"),
                              nullptr, 0, dx, int64_t(N) * D, dxb, int64_t(N) * D, e->blk[L - 1].g2, nullptr, 0, nullptr, 0,
-                             0, B, D, e->eps, s))
+                             0, B, D, e->eps, s, drop_path_scale(e, L - 1, 1), 1))
     return rc;
   }
 
@@ -347,7 +361,7 @@ static int engine_backward(Engine* e, int l_from, int l_to, cudaStream_t s) {
     const BlockPtrs& b = e->blk[l];
     const float* x_in = xs + size_t(2 * l) * TD;
     const float* x_mid = xs + size_t(2 * l + 1) * TD;
-    // MLP branch: dxb holds bf16(gamma2 * dx_out); hpre holds gelu'(fc1 pre-activation) in fp16.  In the last block only
+    // MLP branch: dxb holds bf16(s[l,1] * gamma2 * dx_out); hpre holds gelu'(fc1 pre-activation) in fp16.  In the last block only
     // the CLS rows of dx_out are non-zero (see Engine::cls_last): its MLP input gradients and LayerNorm-2 backward run on
     // those B rows; dx / dxb / dsub of all other rows stay the zeros they were initialised with.
     const bool cls = e->cls_last && l == L - 1;
@@ -362,9 +376,10 @@ static int engine_backward(Engine* e, int l_from, int l_to, cudaStream_t s) {
     void* dsub = dsub0 ? dsub0 + ((side && (l & 1)) ? dsub_slot : 0) : nullptr;
     if (side && dsub && l + 2 <= l_from) APLA_CUDA(cudaStreamWaitEvent(s, e->ev_done[l + 2], 0));
     if (cls && dsub) APLA_CUDA(cudaMemsetAsync(dsub, 0, dsub_bytes, s));
-    // dx_mid = dx_out + LN2'(dln); dxb = bf16(gamma1 * dx_mid); dsub = its APLA columns
+    // dx_mid = dx_out + LN2'(dln); dxb = bf16(s[l,0] * gamma1 * dx_mid); dsub = its APLA columns
     if (int rc = layernorm_bwd(dln, sD, x_mid, sD, b.ln2w, dx, sD, dx, sD, dxb, sD, b.g1, dsub,
-                               cls ? int64_t(N) * e->r_pad : e->r_pad, idx + size_t(l) * r, r, e->r_pad, R, D, e->eps, s))
+                               cls ? int64_t(N) * e->r_pad : e->r_pad, idx + size_t(l) * r, r, e->r_pad, R, D, e->eps, s,
+                               drop_path_scale(e, l, 0), cls ? 1 : N))
       return rc;
     // APLA weight gradient: only the trainable rows of the projection (appla_attn.py:64,70-74)
     float* dW1 = grads + ar.w1 + size_t(l) * r * D;
@@ -402,9 +417,9 @@ static int engine_backward(Engine* e, int l_from, int l_to, cudaStream_t s) {
                          nullptr, D, s, 0))
       return rc;
     if (side && e->full_rows) APLA_CUDA(cudaStreamWaitEvent(s, e->ev_done[l], 0));   // its weight gradient reads dxb
-    // dx_in = dx_mid + LN1'(dln); dxb = bf16(gamma2[l-1] * dx_in) feeds block l-1's MLP branch
+    // dx_in = dx_mid + LN1'(dln); dxb = bf16(s[l-1,1] * gamma2[l-1] * dx_in) feeds block l-1's MLP branch
     if (int rc = layernorm_bwd(dln, D, x_in, D, b.ln1w, dx, D, dx, D, dxb, D, e->blk[l - 1].g2, nullptr, 0, nullptr, 0, 0,
-                               T, D, e->eps, s))
+                               T, D, e->eps, s, drop_path_scale(e, l - 1, 1), N))
       return rc;
   }
   // join: the side stream is serial, so the last block's event covers every weight gradient of this range

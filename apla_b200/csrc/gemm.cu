@@ -398,9 +398,26 @@ int gemm_tn(int epi, const void* A, const void* B, int M, int N, int K, int lda,
   return 1;
 }
 
+int gemm_resid_scaled(const void* A, const void* B, int M, int N, int K, int lda, int ldb, float* out, const float* bias,
+                      const float* gamma, const float* resid, int ldo, const float* row_scale, int rows_per_scale,
+                      cudaStream_t stream) {
+  APLA_CHECK(M > 0 && N > 0 && K > 0, "gemm_resid_scaled: empty problem %dx%dx%d", M, N, K);
+  APLA_CHECK(N % 32 == 0, "gemm_resid_scaled: N=%d must be a multiple of 32", N);
+  APLA_CHECK(K % 8 == 0 && lda % 8 == 0 && ldb % 8 == 0 && ldo % 8 == 0,
+             "gemm_resid_scaled: K/lda/ldb/ldo (%d/%d/%d/%d) must be multiples of 8", K, lda, ldb, ldo);
+  APLA_CHECK(resid != nullptr && row_scale != nullptr && rows_per_scale >= 1,
+             "gemm_resid_scaled: needs the residual, the row scales and rows_per_scale >= 1 (got %d)", rows_per_scale);
+  static const int impl = [] { const char* e = getenv("APLA_GEMM_IMPL"); return e ? atoi(e) : 2; }();
+  APLA_CHECK(impl == 2, "gemm_resid_scaled: the row-scaled residual epilogue exists in the 2-CTA kernel only; "
+             "APLA_GEMM_IMPL=%d selects the 1-CTA kernel", impl);
+  const char* e = getenv("APLA_GEMM_BN");
+  return gemm2_resid_scaled(A, B, M, N, K, lda, ldb, out, bias, gamma, resid, ldo, row_scale, rows_per_scale, stream,
+                            e ? atoi(e) : 0);
+}
+
 int gemm_resid_ln(const void* A, const void* B, int M, int N, int K, int lda, int ldb, float* out, const float* bias,
                   const float* gamma, const float* resid, int ldo, const float* ln_w, const float* ln_b, void* ln_out,
-                  int ld_ln, float eps, cudaStream_t stream, int fuse_mode) {
+                  int ld_ln, float eps, cudaStream_t stream, int fuse_mode, const float* row_scale, int rows_per_scale) {
   // fuse_mode: 1 = one launch, 0 = two launches, < 0 = default, which is one launch only with APLA_GEMM_LN_FUSE=1.  Measured on the C2 step (B200, 50 steps): 8.69 ms fused against 7.93 ms with
   // the two launches -- results bit-identical, but the LayerNorm of a slab lands on the epilogue warps of whichever CTA
   // finishes the slab's last column tile, and those warps are what the K = 768 residual GEMM is already bound by (tensor
@@ -408,6 +425,13 @@ int gemm_resid_ln(const void* A, const void* B, int M, int N, int K, int lda, in
   static const bool fuse = [] { const char* e = getenv("APLA_GEMM_LN_FUSE"); return e && atoi(e) != 0; }();
   static const int impl = [] { const char* e = getenv("APLA_GEMM_IMPL"); return e ? atoi(e) : 2; }();
   const bool want = fuse_mode < 0 ? fuse : fuse_mode != 0;
+  if (row_scale) {
+    APLA_CHECK(!want, "gemm_resid_ln: the one-launch residual + LayerNorm epilogue (APLA_GEMM_LN_FUSE=1) has no row-scaled "
+               "form; unset APLA_GEMM_LN_FUSE to train with drop path");
+    if (int rc = gemm_resid_scaled(A, B, M, N, K, lda, ldb, out, bias, gamma, resid, ldo, row_scale, rows_per_scale, stream))
+      return rc;
+    return layernorm_fwd(out, ldo, ln_w, ln_b, ln_out, ld_ln, M, N, eps, stream);
+  }
   if (want && impl == 2 && gemm2_resid_ln_supported(N) && K % 8 == 0 && lda % 8 == 0 && ldb % 8 == 0 && ldo % 8 == 0)
     return gemm2_resid_ln(A, B, M, N, K, lda, ldb, out, bias, gamma, resid, ldo, ln_w, ln_b, ln_out, ld_ln, eps, stream);
   if (int rc = gemm_tn(EPI_RESID, A, B, M, N, K, lda, ldb, out, nullptr, bias, gamma, resid, ldo, stream, 0)) return rc;

@@ -20,6 +20,9 @@
 //                    column tile of a 128-row slab (a self-resetting arrival counter per slab in global memory)
 //                    re-reads the slab -- still in L2 -- and writes bf16((x - mean) * rstd * w + b), the A operand of
 //                    the next GEMM.  Same arithmetic as ln_fwd_kernel (rowwise.cu), minus its launch and its DRAM pass.
+//   EPI_RESID_SCALED  out_f32 = aux_f32[m,n] + row_scale[m / rows_per_scale] * gamma[n] * (acc + bias[n]): EPI_RESID
+//                    with one scale per group of rows (stochastic depth: per image; 0 or 1/keep), folded into gamma, so
+//                    a scale of 1 gives EPI_RESID's bits
 //   EPI_DELTA  out_bf16 = acc;  rowstat[m, n/64] = sum over the 64-wide head of bf16(acc) * aux_bf16[m, n]
 //              (attention-projection dgrad fused with FlashAttention's delta = rowsum(dO * O); one staging chunk is
 //              exactly one head and one thread owns one row of it, so the reduction needs no shuffles).
@@ -73,6 +76,7 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// arguments of the epilogues beyond the GEMM's: the LayerNorm of EPI_RESID_LN, the row scales of EPI_RESID_SCALED
 struct LnArgs {
   const float* x;   // the fp32 output of this GEMM (read back by generic loads)
   int64_t ldx;
@@ -82,6 +86,8 @@ struct LnArgs {
   int* counters;   // [row slabs of 128] arrival counters, zero between launches (the last arriver resets its slab's)
   int ld;
   float eps;
+  const float* row_scale;   // EPI_RESID_SCALED: row m is scaled by row_scale[m / rows_per_scale]
+  int rows_per_scale;
 };
 
 // LayerNorm of `nrows` consecutive rows (two at a time: the loads of both are in flight together) by one warp;
@@ -162,7 +168,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ 
     tma_prefetch_desc(&tma_b);
     tma_prefetch_desc(&tma_out);
     if constexpr (EPI == EPI_BIAS_GELU || EPI == EPI_BIAS_GELU_D) tma_prefetch_desc(&tma_out2);
-    if constexpr (EPI == EPI_RESID || EPI == EPI_RESID_LN || EPI == EPI_GELU_BWD || EPI == EPI_DELTA || EPI == EPI_MUL_F16) tma_prefetch_desc(&tma_aux);
+    if constexpr (EPI == EPI_RESID || EPI == EPI_RESID_LN || EPI == EPI_RESID_SCALED || EPI == EPI_GELU_BWD || EPI == EPI_DELTA || EPI == EPI_MUL_F16) tma_prefetch_desc(&tma_aux);
     for (int s = 0; s < kStages; ++s) {
       mbar_init(&full[s], 1);
       mbar_init(&empty[s], 1);
@@ -237,10 +243,14 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ 
   } else {
     // ===================== epilogue warps (both CTAs) =====================
     constexpr bool kLN = (EPI == EPI_RESID_LN);
-    constexpr bool kF32 = (EPI == EPI_RESID || kLN || EPI == EPI_RED);
-    constexpr bool kAux = (EPI == EPI_RESID || kLN || EPI == EPI_GELU_BWD || EPI == EPI_DELTA || EPI == EPI_MUL_F16);
+    constexpr bool kF32 = (EPI == EPI_RESID || kLN || EPI == EPI_RED || EPI == EPI_RESID_SCALED);
+    constexpr bool kAux = (EPI == EPI_RESID || kLN || EPI == EPI_RESID_SCALED || EPI == EPI_GELU_BWD || EPI == EPI_DELTA ||
+                           EPI == EPI_MUL_F16);
     constexpr bool kBias = (EPI != EPI_GELU_BWD && EPI != EPI_DELTA && EPI != EPI_MUL_F16);
     constexpr bool kTwoOut = (EPI == EPI_BIAS_GELU || EPI == EPI_BIAS_GELU_D);
+    // the bias is read at its use, not one sub-load ahead: the prefetch holds 32 registers, which the LayerNorm and the
+    // row scale need (without this, both spill)
+    constexpr bool kBiasAtUse = (kLN || EPI == EPI_RESID_SCALED);
     // the GELU epilogues in packed fp32 add the bias inside gelu_erf_both_x2, not to the accumulator beforehand
     constexpr bool kGeluX2 = (EPI == EPI_BIAS_GELU_D || EPI == EPI_BIAS_GELU_G);
     // columns per chunk: one 128-byte staging row, except the two-output GELU epilogue which packs a 64-byte row of
@@ -325,7 +335,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ 
       }
       if (nvalid > 0) {
         tmem_ld_32x32(t_base, v[0]);
-        if constexpr (kBias && !kLN) {   // (EPI_RESID_LN reads the bias at its use: it needs the 32 registers)
+        if constexpr (kBias && !kBiasAtUse) {
           if (bias) {
 #pragma unroll
             for (int i = 0; i < 8; ++i) bb[i] = __ldg(reinterpret_cast<const float4*>(bias + n0 + half * CW) + i);
@@ -389,7 +399,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ 
               }
             }
             if (bias) {
-              if constexpr (kLN) {
+              if constexpr (kBiasAtUse) {
 #pragma unroll
                 for (int i = 0; i < 8; ++i) {
                   const float4 t4 = __ldg(reinterpret_cast<const float4*>(bias + col) + i);
@@ -402,7 +412,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ 
                   x[4 * i] += t4.x; x[4 * i + 1] += t4.y; x[4 * i + 2] += t4.z; x[4 * i + 3] += t4.w;
                 }
               }
-              if (!kLN && idx + 1 < NSUB && idx + 1 < nvalid) {
+              if (!kBiasAtUse && idx + 1 < NSUB && idx + 1 < nvalid) {
                 const int j1 = (idx + 1) / SUBS, s1 = (idx + 1) % SUBS;
                 const float4* b4 = reinterpret_cast<const float4*>(bias + n0 + (half + 2 * j1) * CW + s1 * 32);
 #pragma unroll
@@ -475,13 +485,22 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ 
               sts128(stg_addr(buf, lane, c), __float_as_uint(g.x * x[4 * c]), __float_as_uint(g.y * x[4 * c + 1]),
                      __float_as_uint(g.z * x[4 * c + 2]), __float_as_uint(g.w * x[4 * c + 3]));
             }
-          } else if constexpr (EPI == EPI_RESID || EPI == EPI_RESID_LN) {
+          } else if constexpr (EPI == EPI_RESID || EPI == EPI_RESID_LN || EPI == EPI_RESID_SCALED) {
             const float4* g4 = reinterpret_cast<const float4*>(gamma ? gamma + col : nullptr);
+            // EPI_RESID_SCALED: the scale of this thread's row (lane = row of the slab), read at its use -- holding it
+            // across the tile costs a register this kernel does not have
+            [[maybe_unused]] float rscale = 0.f;
+            if constexpr (EPI == EPI_RESID_SCALED) {
+              if (row0 + lane < M) rscale = __ldg(ln.row_scale + (row0 + lane) / ln.rows_per_scale);
+            }
 #pragma unroll
             for (int c = 0; c < 8; ++c) {
               const uint32_t a = stg_addr(buf, lane, c);
               const uint4 rv = lds128(a);
-              const float4 g = gamma ? __ldg(g4 + c) : make_float4(1.f, 1.f, 1.f, 1.f);
+              float4 g = gamma ? __ldg(g4 + c) : make_float4(1.f, 1.f, 1.f, 1.f);
+              if constexpr (EPI == EPI_RESID_SCALED) {
+                g.x *= rscale; g.y *= rscale; g.z *= rscale; g.w *= rscale;
+              }
               sts128(a, __float_as_uint(__uint_as_float(rv.x) + g.x * x[4 * c]),
                      __float_as_uint(__uint_as_float(rv.y) + g.y * x[4 * c + 1]),
                      __float_as_uint(__uint_as_float(rv.z) + g.z * x[4 * c + 2]),
@@ -560,7 +579,7 @@ static int launch(const void* A, const void* B, int M, int N, int K, int lda, in
   CUtensorMap ta, tb, to, to2, tx;
   if (int rc = make_tmap_2d(&ta, A, 2, M, K, lda, BM, BK, true)) return rc;
   if (int rc = make_tmap_2d(&tb, B, 2, N, K, ldb, BN / 2, BK, true)) return rc;
-  constexpr int oelt = (EPI == EPI_RESID || EPI == EPI_RESID_LN || EPI == EPI_RED) ? 4 : 2;
+  constexpr int oelt = (EPI == EPI_RESID || EPI == EPI_RESID_LN || EPI == EPI_RESID_SCALED || EPI == EPI_RED) ? 4 : 2;
   if (EPI == EPI_BIAS_GELU || EPI == EPI_BIAS_GELU_D) {
     if (int rc = make_tmap_2d_sw(&to, out, 2, M, N, ldo, 32, 32, 64)) return rc;
     if (int rc = make_tmap_2d_sw(&to2, out2, 2, M, N, ldo, 32, 32, 64)) return rc;
@@ -569,7 +588,8 @@ static int launch(const void* A, const void* B, int M, int N, int K, int lda, in
     to2 = to;
   }
   tx = to;
-  if (EPI == EPI_RESID || EPI == EPI_RESID_LN || EPI == EPI_GELU_BWD || EPI == EPI_DELTA || EPI == EPI_MUL_F16)
+  if (EPI == EPI_RESID || EPI == EPI_RESID_LN || EPI == EPI_RESID_SCALED || EPI == EPI_GELU_BWD || EPI == EPI_DELTA ||
+      EPI == EPI_MUL_F16)
     if (int rc = make_tmap_2d(&tx, aux, oelt, M, N, ldo, 32, 128 / oelt, true)) return rc;
   auto kern = gemm2_kernel<BN, EPI>;
   static bool attr_set = false;
@@ -625,6 +645,18 @@ int gemm2_resid_ln(const void* A, const void* B, int M, int N, int K, int lda, i
   }
   g2::LnArgs ln{out, int64_t(ldo), ln_w, ln_b, reinterpret_cast<__nv_bfloat16*>(ln_out), counters[dev], ld_ln, eps};
   return g2::launch<256, EPI_RESID_LN>(A, B, M, N, K, lda, ldb, out, nullptr, bias, gamma, resid, ldo, stream, ln);
+}
+
+int gemm2_resid_scaled(const void* A, const void* B, int M, int N, int K, int lda, int ldb, float* out, const float* bias,
+                       const float* gamma, const float* resid, int ldo, const float* row_scale, int rows_per_scale,
+                       cudaStream_t stream, int bn) {
+  g2::LnArgs ex{};
+  ex.row_scale = row_scale;
+  ex.rows_per_scale = rows_per_scale;
+  if (bn != 128 && bn != 256) bn = g2::pick_bn(M, N);
+  if (bn == 256)
+    return g2::launch<256, EPI_RESID_SCALED>(A, B, M, N, K, lda, ldb, out, nullptr, bias, gamma, resid, ldo, stream, ex);
+  return g2::launch<128, EPI_RESID_SCALED>(A, B, M, N, K, lda, ldb, out, nullptr, bias, gamma, resid, ldo, stream, ex);
 }
 
 int gemm2_tn(int epi, const void* A, const void* B, int M, int N, int K, int lda, int ldb, void* out, void* out2,

@@ -6,7 +6,7 @@
 namespace apla {
 
 enum { EPI_BIAS = 0, EPI_BIAS_GELU = 1, EPI_RESID = 2, EPI_GELU_BWD = 3, EPI_F32_T = 4, EPI_DELTA = 5, EPI_BIAS_GELU_D = 6,
-       EPI_MUL_F16 = 7, EPI_RED = 8, EPI_RESID_LN = 9, EPI_BIAS_GELU_G = 10 };
+       EPI_MUL_F16 = 7, EPI_RED = 8, EPI_RESID_LN = 9, EPI_BIAS_GELU_G = 10, EPI_RESID_SCALED = 11 };
 
 // gemm.cu
 int gemm_tn(int epi, const void* A, const void* B, int M, int N, int K, int lda, int ldb, void* out, void* out2,
@@ -16,10 +16,20 @@ int gemm2_tn(int epi, const void* A, const void* B, int M, int N, int K, int lda
 int gemm_wgrad_nt(const void* A, const void* B, int M, int N, int K, int lda, int ldb, float* dW, int ldw,
                   const int* rowmap, int n_valid, cudaStream_t stream);
 // out_f32 = resid + gamma * (A B^T + bias) and ln_out_bf16 = LayerNorm(out_f32): one launch when the 2-CTA kernel covers
-// the width (gemm2.cu, EPI_RESID_LN), otherwise the residual GEMM followed by layernorm_fwd
+// the width (gemm2.cu, EPI_RESID_LN), otherwise the residual GEMM followed by layernorm_fwd.  With row_scale set, the
+// branch of row m is scaled by row_scale[m / rows_per_scale] (gemm_resid_scaled), always in the two-launch form.
 int gemm_resid_ln(const void* A, const void* B, int M, int N, int K, int lda, int ldb, float* out, const float* bias,
                   const float* gamma, const float* resid, int ldo, const float* ln_w, const float* ln_b, void* ln_out,
-                  int ld_ln, float eps, cudaStream_t stream, int fuse_mode = -1);
+                  int ld_ln, float eps, cudaStream_t stream, int fuse_mode = -1, const float* row_scale = nullptr,
+                  int rows_per_scale = 1);
+// out_f32 = resid + row_scale[m / rows_per_scale] * gamma * (A B^T + bias): the residual epilogue with a per-row-group
+// scale (stochastic depth), 2-CTA kernel only (gemm2.cu, EPI_RESID_SCALED)
+int gemm_resid_scaled(const void* A, const void* B, int M, int N, int K, int lda, int ldb, float* out, const float* bias,
+                      const float* gamma, const float* resid, int ldo, const float* row_scale, int rows_per_scale,
+                      cudaStream_t stream);
+int gemm2_resid_scaled(const void* A, const void* B, int M, int N, int K, int lda, int ldb, float* out, const float* bias,
+                       const float* gamma, const float* resid, int ldo, const float* row_scale, int rows_per_scale,
+                       cudaStream_t stream, int bn);
 bool gemm2_resid_ln_supported(int N);
 int gemm2_resid_ln(const void* A, const void* B, int M, int N, int K, int lda, int ldb, float* out, const float* bias,
                    const float* gamma, const float* resid, int ldo, const float* ln_w, const float* ln_b, void* ln_out,
@@ -63,9 +73,11 @@ int attn_probs(const void* qkv, const float* lse, float* probs, int B, int N, in
 // rowwise.cu
 int layernorm_fwd(const float* x, int64_t ldx, const float* w, const float* b, void* y, int64_t ldy, int rows, int D,
                   float eps, cudaStream_t stream);
+// row_scale set: dxb and sub of row t are also scaled by row_scale[t / rows_per_scale] (dx is not); D % 128 == 0 only
 int layernorm_bwd(const void* dy, int64_t ld_dy, const float* x, int64_t ldx, const float* w, const float* dres,
                   int64_t ld_dres, float* dx, int64_t ld_dx, void* dxb, int64_t ld_dxb, const float* gamma, void* sub,
-                  int64_t ld_sub, const int* idx, int r, int r_pad, int rows, int D, float eps, cudaStream_t stream);
+                  int64_t ld_sub, const int* idx, int r, int r_pad, int rows, int D, float eps, cudaStream_t stream,
+                  const float* row_scale = nullptr, int rows_per_scale = 1);
 int gather_cols(const void* dy, int64_t ld, void* sub, int64_t ld_sub, const int* idx, int r, int r_pad, int rows,
                 cudaStream_t stream);
 int ls_cast(const float* x, int64_t ldx, const float* gamma, void* out, int64_t ldo, int rows, int D,

@@ -64,20 +64,24 @@ ln_fwd_kernel(const float* __restrict__ x, int64_t ldx, const float* __restrict_
 //   dxb     = bf16(gamma * dx)                    -> A operand of the next dgrad GEMM (LayerScale folded in)
 //   sub[j]  = bf16(gamma[idx[j]] * dx[idx[j]])    -> compact gathered columns for the APLA weight gradient
 // mean / rstd are recomputed from x (the row is read anyway).
+// kScaled (ln_bwd_scaled_kernel): dxb and sub are also multiplied by the row's scale row_scale[row / rows_per_scale] --
+// the stochastic-depth mask of the branch that reads them; dx, the residual-stream gradient, is not.
 // ------------------------------------------------------------------------------------------------
-template <int NV>
-__global__ void __launch_bounds__(256)
-ln_bwd_kernel(const __nv_bfloat16* __restrict__ dy, int64_t ld_dy, const float* __restrict__ x, int64_t ldx,
-              const float* __restrict__ w, const float* dres, int64_t ld_dres, float* dx, int64_t ld_dx,
-              __nv_bfloat16* __restrict__ dxb, int64_t ld_dxb, const float* __restrict__ gamma,
-              __nv_bfloat16* __restrict__ sub, int64_t ld_sub, const int* __restrict__ idx, int r, int r_pad, int rows,
-              float eps) {
+template <int NV, bool kScaled>
+__device__ __forceinline__ void
+ln_bwd_row(const __nv_bfloat16* __restrict__ dy, int64_t ld_dy, const float* __restrict__ x, int64_t ldx,
+           const float* __restrict__ w, const float* dres, int64_t ld_dres, float* dx, int64_t ld_dx,
+           __nv_bfloat16* __restrict__ dxb, int64_t ld_dxb, const float* __restrict__ gamma,
+           __nv_bfloat16* __restrict__ sub, int64_t ld_sub, const int* __restrict__ idx, int r, int r_pad, int rows,
+           float eps, const float* __restrict__ row_scale, int rows_per_scale) {
   constexpr int D = NV * 128;
   extern __shared__ float srow[];  // [warps][D], only used when sub != nullptr
   const int wib = threadIdx.x >> 5;
   const int row = blockIdx.x * (blockDim.x >> 5) + wib;
   const int lane = threadIdx.x & 31;
   if (row >= rows) return;
+  [[maybe_unused]] float rscale = 1.f;
+  if constexpr (kScaled) rscale = __ldg(row_scale + row / rows_per_scale);
   const float4* xr = reinterpret_cast<const float4*>(x + row * ldx);
   const uint2* dyr = reinterpret_cast<const uint2*>(dy + row * ld_dy);
   const float4* rr = dres ? reinterpret_cast<const float4*>(dres + row * ld_dres) : nullptr;
@@ -134,6 +138,9 @@ ln_bwd_kernel(const __nv_bfloat16* __restrict__ dy, int64_t ld_dy, const float* 
         const float4 gm = __ldg(reinterpret_cast<const float4*>(gamma) + lane + 32 * i);
         o.x *= gm.x; o.y *= gm.y; o.z *= gm.z; o.w *= gm.w;
       }
+      if constexpr (kScaled) {
+        o.x *= rscale; o.y *= rscale; o.z *= rscale; o.w *= rscale;
+      }
       if (outb) outb[lane + 32 * i] = make_uint2(pack_bf16(o.x, o.y), pack_bf16(o.z, o.w));
       if (sub) reinterpret_cast<float4*>(sr)[lane + 32 * i] = o;
     }
@@ -143,6 +150,28 @@ ln_bwd_kernel(const __nv_bfloat16* __restrict__ dy, int64_t ld_dy, const float* 
     __nv_bfloat16* so = sub + row * ld_sub;
     for (int j = lane; j < r_pad; j += 32) so[j] = __float2bfloat16_rn(j < r ? sr[__ldg(idx + j)] : 0.f);
   }
+}
+
+template <int NV>
+__global__ void __launch_bounds__(256)
+ln_bwd_kernel(const __nv_bfloat16* __restrict__ dy, int64_t ld_dy, const float* __restrict__ x, int64_t ldx,
+              const float* __restrict__ w, const float* dres, int64_t ld_dres, float* dx, int64_t ld_dx,
+              __nv_bfloat16* __restrict__ dxb, int64_t ld_dxb, const float* __restrict__ gamma,
+              __nv_bfloat16* __restrict__ sub, int64_t ld_sub, const int* __restrict__ idx, int r, int r_pad, int rows,
+              float eps) {
+  ln_bwd_row<NV, false>(dy, ld_dy, x, ldx, w, dres, ld_dres, dx, ld_dx, dxb, ld_dxb, gamma, sub, ld_sub, idx, r, r_pad,
+                        rows, eps, nullptr, 1);
+}
+
+template <int NV>
+__global__ void __launch_bounds__(256)
+ln_bwd_scaled_kernel(const __nv_bfloat16* __restrict__ dy, int64_t ld_dy, const float* __restrict__ x, int64_t ldx,
+                     const float* __restrict__ w, const float* dres, int64_t ld_dres, float* dx, int64_t ld_dx,
+                     __nv_bfloat16* __restrict__ dxb, int64_t ld_dxb, const float* __restrict__ gamma,
+                     __nv_bfloat16* __restrict__ sub, int64_t ld_sub, const int* __restrict__ idx, int r, int r_pad,
+                     int rows, float eps, const float* __restrict__ row_scale, int rows_per_scale) {
+  ln_bwd_row<NV, true>(dy, ld_dy, x, ldx, w, dres, ld_dres, dx, ld_dx, dxb, ld_dxb, gamma, sub, ld_sub, idx, r, r_pad,
+                       rows, eps, row_scale, rows_per_scale);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -411,13 +440,26 @@ int layernorm_fwd(const float* x, int64_t ldx, const float* w, const float* b, v
 
 int layernorm_bwd(const void* dy, int64_t ld_dy, const float* x, int64_t ldx, const float* w, const float* dres,
                   int64_t ld_dres, float* dx, int64_t ld_dx, void* dxb, int64_t ld_dxb, const float* gamma, void* sub,
-                  int64_t ld_sub, const int* idx, int r, int r_pad, int rows, int D, float eps, cudaStream_t stream) {
+                  int64_t ld_sub, const int* idx, int r, int r_pad, int rows, int D, float eps, cudaStream_t stream,
+                  const float* row_scale, int rows_per_scale) {
   APLA_CHECK(rows > 0, "layernorm_bwd: no rows");
   APLA_CHECK(D > 0 && D % 4 == 0 && D <= 128 * kMaxV4, "layernorm_bwd: D=%d must be a multiple of 4 and <= 1024", D);
   APLA_CHECK(ld_dy % 4 == 0 && ldx % 4 == 0 && ld_dx % 4 == 0 && ld_dres % 4 == 0 && ld_dxb % 4 == 0,
              "layernorm_bwd: leading dimensions must be multiples of 4");
   APLA_CHECK(sub == nullptr || (idx != nullptr && r <= r_pad && r_pad <= ld_sub), "layernorm_bwd: bad gather arguments");
   const int grid = cdiv(rows, 8);
+  if (row_scale) {
+    APLA_CHECK(D % 128 == 0, "layernorm_bwd: the row-scaled backward needs D a multiple of 128, got %d", D);
+    APLA_CHECK(rows_per_scale >= 1, "layernorm_bwd: rows_per_scale=%d must be >= 1", rows_per_scale);
+    const size_t smem = sub ? size_t(8) * D * sizeof(float) : 0;
+    LN_DISPATCH(D / 128, (ln_bwd_scaled_kernel<NV><<<grid, 256, smem, stream>>>(
+                             reinterpret_cast<const __nv_bfloat16*>(dy), ld_dy, x, ldx, w, dres, ld_dres, dx, ld_dx,
+                             reinterpret_cast<__nv_bfloat16*>(dxb), ld_dxb, gamma, reinterpret_cast<__nv_bfloat16*>(sub),
+                             ld_sub, idx, r, r_pad, rows, eps, row_scale, rows_per_scale)));
+    APLA_CUDA(cudaGetLastError());
+    count_launch();
+    return 0;
+  }
   if (D % 128 != 0) {
     ln_bwd_generic_kernel<<<grid, 256, 0, stream>>>(
         reinterpret_cast<const __nv_bfloat16*>(dy), ld_dy, x, ldx, w, dres, ld_dres, dx, ld_dx,

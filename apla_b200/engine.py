@@ -15,13 +15,14 @@ Memory layout in HBM (T = B*N tokens, D embed, L blocks), sized for B=64 ViT-B/1
   qkv[l]    bf16 [T, 3D]  ao[l] bf16 [T, D]  lse[l] fp32 [T, H]  hpre[l] fp16 [T, 4D] (gelu' of the fc1 pre-activation)   saved for backward
   ln_out, gelu_out, dx, dxb, dO, dqkv, dsub, delta                                         transients, reused
   params / grads / exp_avg / exp_avg_sq   fp32 arenas [W1 x L | fc.weight | b1 x L | fc.bias]  (one all-reduce)
+  drop_path fp32 [L, 2, B]  stochastic-depth scales of the attention / MLP branch per image (only with a rate > 0)
   infer_*   evaluation workspace of predict / embed / evaluate (eval_batch_size images, allocated on first use): two fp32
             [T_eval, D] residual buffers and one block's transients -- no checkpoints, nothing kept for backward
 """
 from __future__ import annotations
 
 import math
-from typing import Dict, List, Optional
+from typing import Dict, List, Optional, Tuple
 
 import os
 
@@ -29,6 +30,7 @@ import torch
 import torch.nn as nn
 
 from ._lib import LIB, ptr, require_device, stream
+from .apla.apla_block import _drop_rate as _rate
 
 BF16, F32 = torch.bfloat16, torch.float32
 
@@ -64,6 +66,46 @@ def criterion_code(criterion) -> int:
     raise ValueError(f"criterion {type(criterion).__name__} is not supported; " + supported)
 
 
+def drop_path_rates(model) -> List[Tuple[float, float]]:
+    """The stochastic-depth rates (p_attn, p_mlp) of every block of `model.backbone`: `blk.drop_path.drop_prob` for both
+    branches (the reference's Block, vit.py), or timm's `drop_path1` / `drop_path2`; nn.Identity is rate 0.  The engine
+    draws the masks itself (one per image, branch and step).  Raises ValueError for what it cannot honour: dropout
+    anywhere (`attn.attn_drop`, `attn.proj_drop`, `mlp.drop`, `backbone.pos_drop` -- it would need RNG inside the kernels),
+    DropPath(scale_by_keep=False), DINOv2's batch-subset stochastic depth (sample_drop_ratio > 0.1) and rates >= 1."""
+    bb = model.backbone
+
+    def no_dropout(name, mod):
+        p = _rate(mod)
+        if p > 0:
+            raise ValueError(f"{name} has dropout rate {p}: the step engine cannot honour dropout (--dr / --adr); set it to "
+                             "0 (stochastic depth, drop_path_rate / --dpr, is supported)")
+
+    no_dropout("backbone.pos_drop", getattr(bb, "pos_drop", None))
+    rates = []
+    for l, blk in enumerate(bb.blocks):
+        pre = f"backbone.blocks.{l}."
+        no_dropout(pre + "attn.attn_drop", getattr(blk.attn, "attn_drop", None))
+        no_dropout(pre + "attn.proj_drop", getattr(blk.attn, "proj_drop", None))
+        for name in ("drop", "drop1", "drop2"):
+            no_dropout(pre + "mlp." + name, getattr(blk.mlp, name, None))
+        if float(getattr(blk, "sample_drop_ratio", 0.0) or 0.0) > 0.1:
+            raise ValueError(f"{pre[:-1]}: sample_drop_ratio > 0.1 selects DINOv2's batch-subset stochastic depth, which "
+                             "the step engine cannot honour")
+        if hasattr(blk, "drop_path1") or hasattr(blk, "drop_path2"):
+            mods = (getattr(blk, "drop_path1", None), getattr(blk, "drop_path2", None))
+        else:
+            mods = (getattr(blk, "drop_path", None),) * 2
+        for m in mods:
+            if getattr(m, "scale_by_keep", True) is False:
+                raise ValueError(f"{pre[:-1]}: DropPath(scale_by_keep=False) is not supported; the engine scales the kept "
+                                 "samples by 1 / keep as the reference's drop_path does")
+        pair = (_rate(mods[0]), _rate(mods[1]))
+        if not all(0.0 <= p < 1.0 for p in pair):
+            raise ValueError(f"{pre[:-1]}: drop-path rates {pair} outside [0, 1)")
+        rates.append(pair)
+    return rates
+
+
 def interpolate_pos_table(pos_embed: torch.Tensor, npatch: int) -> torch.Tensor:
     """Bicubic resize of a [1, 1+n0, D] position table to an npatch grid (vit.py:421-437); done ONCE at engine
     construction because pos_embed is frozen (the reference recomputes it every forward, SURVEY.md K21)."""
@@ -85,6 +127,8 @@ class FineTuneEngine:
                  eval_batch_size: Optional[int] = None, criterion=None):
         # the trainer's loss (`criterion=self.criterion`): 0 = cross-entropy, 1 = BCE-with-logits (multi-label)
         self.criterion = criterion_code(criterion)
+        # stochastic depth per block and branch (the reference's --dpr); models with dropout are refused here
+        self.drop_path = drop_path_rates(model)
         require_device()
         # Only norm(x)[:, 0] of the last block reaches the head (vit.py:417-419): its projection, LayerNorm 2, MLP and
         # their input gradients run on the CLS rows only.  False = every token (identical results, for A/B checks).
@@ -113,6 +157,13 @@ class FineTuneEngine:
         if self.eval_batch_size < 1:
             raise ValueError("eval_batch_size must be >= 1")
         self._infer_ws: Optional[Dict[str, torch.Tensor]] = None
+        # the drop-path masks of every training forward come from this generator, on the host; seeded per rank so that
+        # ranks drop different images, as the reference's per-process RNG does
+        rank = torch.distributed.get_rank(process_group) if self._dist_on() else 0
+        self._dp_gen = torch.Generator().manual_seed((torch.initial_seed() + 1_000_003 * rank) % 2 ** 63)
+        self._dp_dev: Optional[torch.Tensor] = None
+        # CPU fp32 [L, 2, n]: the scales (0 or 1 / keep) the last training forward applied; None when every rate is 0
+        self.last_drop_path_scales: Optional[torch.Tensor] = None
         self._build(model, batch_size, img_size)
 
     # ------------------------------------------------------------------------------------------------------------
@@ -301,6 +352,11 @@ class FineTuneEngine:
         self._hyper_dev = self._new(3, dtype=F32, zero=True)
         if self.use_graph:
             self._set("hyper", self._hyper_dev)
+        if any(p > 0 for pair in self.drop_path for p in pair):
+            self._dp_keep = 1.0 - torch.tensor(self.drop_path, dtype=torch.float64)     # [L, 2]
+            self._dp_dev = self._new(L, 2, B, dtype=F32)
+            self._dp_dev.fill_(1.0)
+            self._set("drop_path", self._dp_dev)
         self.images_dev = self._new(B, 3, img, img, dtype=F32)
         self.labels_dev = self._new(B, dtype=torch.int64)
         self._ar_stream = torch.cuda.Stream(device=self.device) if self.world > 1 else None
@@ -474,14 +530,33 @@ class FineTuneEngine:
         LIB.call("apla_engine_forward_n", self._handle, ptr(images), n, None if soft else ptr(labels),
                  ptr(labels) if soft else None, inv, inv, stream())
 
+    def _draw_drop_path(self, n: int) -> torch.Tensor:
+        """-> CPU fp32 [L, 2, n] stochastic-depth scales: image b keeps branch (l, j) with probability keep = 1 - p[l][j]
+        (an independent draw per image, branch and call, as vit.py's drop_path) and is then scaled by 1 / keep."""
+        keep = self._dp_keep[:, :, None]
+        u = torch.rand(self.shape["L"], 2, n, generator=self._dp_gen, dtype=torch.float64)
+        return ((u < keep).double() / keep).float()
+
+    def _push_drop_path(self, n: int):
+        """New masks for the training forward about to run -> the device buffer (stream-ordered, like _push_hyper)."""
+        scales = self._draw_drop_path(n)
+        self.last_drop_path_scales = scales
+        full = torch.ones(self.shape["L"], 2, self.shape["B"], dtype=F32)
+        full[:, :, :n] = scales
+        # a fresh pageable tensor: its bytes are staged at call time (see _push_hyper)
+        self._dp_dev.copy_(full, non_blocking=True)
+
     def forward(self, images: torch.Tensor, labels: Optional[torch.Tensor] = None) -> torch.Tensor:
         """images fp32 [n,3,S,S] (1 <= n <= B) on the engine's device -> logits fp32 [n,C], a view of the first n rows of
         `self.logits` (and loss / dlogits when labels are given: int64 [n] class indices or fp32 [n, C] probabilities;
         on a BCE-with-logits engine fp32 [n, C] multi-label targets, with the mean over the n*C elements).
-        The next backward() runs over the same n images."""
+        The next backward() runs over the same n images.  With drop path (a model built with drop_path_rate > 0) this is
+        the training forward: it draws new masks (`last_drop_path_scales`); `predict` is the evaluation forward."""
         n = self._check_inputs(images, labels)
         images = images.contiguous()
         labels = labels.contiguous() if labels is not None else None
+        if self._dp_dev is not None:
+            self._push_drop_path(n)
         self._launch_forward(images, labels, n)
         return self.logits if n == self.shape["B"] else self.logits[:n]
 
@@ -615,6 +690,9 @@ class FineTuneEngine:
             self._graph_keep = getattr(self, "_graph_keep", []) + [(images, labels)]   # keep the buffers alive
         self.step_count += 1
         self._push_hyper()
+        if self._dp_dev is not None:
+            # drawn outside any capture: the graphs read the buffer, every replay gets new masks
+            self._push_drop_path(int(images.shape[0]))
         if self.world == 1 or self._peer is not None:
             g[0].replay()
             return self.loss

@@ -91,12 +91,33 @@ class ChannelScale(nn.Module):
         return x * self.gamma
 
 
+def drop_path(x, drop_prob: float = 0.0, training: bool = False):
+    """Stochastic depth (vit.py drop_path): in training, every sample of the batch is kept with probability
+    keep = 1 - drop_prob -- one draw per sample and call -- and the kept ones are scaled by 1 / keep."""
+    if drop_prob == 0.0 or not training:
+        return x
+    keep = 1.0 - drop_prob
+    mask = (keep + torch.rand((x.shape[0],) + (1,) * (x.ndim - 1), dtype=x.dtype, device=x.device)).floor_()
+    return x.div(keep) * mask
+
+
+class DropPath(nn.Module):
+    def __init__(self, drop_prob: Optional[float] = None):
+        super().__init__()
+        self.drop_prob = drop_prob
+
+    def forward(self, x):
+        return drop_path(x, self.drop_prob, self.training)
+
+
 class EncoderBlock(nn.Module):
     def __init__(self, dim: int, num_heads: int, mlp_ratio: float, qkv_bias: bool, eps: float,
-                 layerscale: Optional[float]):
+                 layerscale: Optional[float], drop_path_rate: float = 0.0):
         super().__init__()
         self.norm1 = nn.LayerNorm(dim, eps=eps)
         self.attn = SoftmaxAttention(dim, num_heads, qkv_bias)
+        # one module for both branches, as the reference's Block: each call draws its own masks
+        self.drop_path = DropPath(drop_path_rate) if drop_path_rate > 0.0 else nn.Identity()
         self.norm2 = nn.LayerNorm(dim, eps=eps)
         self.mlp = FeedForward(dim, int(dim * mlp_ratio))
         self.ls1 = ChannelScale(dim, layerscale) if layerscale is not None else nn.Identity()
@@ -105,8 +126,8 @@ class EncoderBlock(nn.Module):
     def forward(self, x):
         y = self.attn(self.norm1(x))
         y = y[0] if isinstance(y, tuple) else y
-        x = x + self.ls1(y)
-        return x + self.ls2(self.mlp(self.norm2(x)))
+        x = x + self.drop_path(self.ls1(y))
+        return x + self.drop_path(self.ls2(self.mlp(self.norm2(x))))
 
 
 class PatchProjection(nn.Module):
@@ -122,7 +143,7 @@ class PatchProjection(nn.Module):
 
 class HostViT(nn.Module):
     def __init__(self, arch: VitArch, img_size: int = 518, patch_size: int = 14, layerscale: Optional[float] = 1.0,
-                 eps: float = 1e-6):
+                 eps: float = 1e-6, drop_path_rate: float = 0.0):
         super().__init__()
         D = arch.embed_dim
         self.arch = arch
@@ -130,8 +151,11 @@ class HostViT(nn.Module):
         self.patch_embed = PatchProjection(img_size, patch_size, D)
         self.cls_token = nn.Parameter(torch.zeros(1, 1, D))
         self.pos_embed = nn.Parameter(torch.zeros(1, self.patch_embed.num_patches + 1, D))
+        # stochastic depth rising linearly over depth (vit.py: dpr = linspace(0, drop_path_rate, depth)); no RNG drawn
+        dpr = [float(p) for p in torch.linspace(0, drop_path_rate, arch.depth)]
         self.blocks = nn.ModuleList(
-            [EncoderBlock(D, arch.num_heads, arch.mlp_ratio, arch.qkv_bias, eps, layerscale) for _ in range(arch.depth)])
+            [EncoderBlock(D, arch.num_heads, arch.mlp_ratio, arch.qkv_bias, eps, layerscale, dpr[i])
+             for i in range(arch.depth)])
         self.norm = nn.LayerNorm(D, eps=eps)
         self.fc = nn.Identity()
         _trunc_normal_(self.pos_embed, 0.02)
@@ -187,12 +211,14 @@ class HostClassifier(nn.Module):
 
 
 def build_classifier(arch: str, *, img_size: int, patch_size: int, n_classes: int, apla_config, is_multi_gpu=False,
-                     attn_class: str = "apla_attn", layerscale: Optional[float] = 1.0, seed: Optional[int] = 0):
-    """Construct backbone -> build_apla -> head in the reference's order (models.py:39-65) on the CPU generator."""
+                     attn_class: str = "apla_attn", layerscale: Optional[float] = 1.0, seed: Optional[int] = 0,
+                     drop_path_rate: float = 0.0):
+    """Construct backbone -> build_apla -> head in the reference's order (models.py:39-65) on the CPU generator.
+    `drop_path_rate` is the reference's --dpr; it changes no weight."""
     from .apla.apla_vit import build_apla
     if seed is not None:
         torch.manual_seed(seed)
     a = ARCHS[arch] if isinstance(arch, str) else arch
-    vit = HostViT(a, img_size=img_size, patch_size=patch_size, layerscale=layerscale)
+    vit = HostViT(a, img_size=img_size, patch_size=patch_size, layerscale=layerscale, drop_path_rate=drop_path_rate)
     vit = build_apla(apla_config, vit, attn_class, is_multi_gpu=is_multi_gpu)
     return HostClassifier(vit, n_classes)

@@ -44,6 +44,15 @@ int apla_gemm_bias_gelu_fwd(const void* A, int lda, const void* W, int ldw, cons
 int apla_gemm_bias_ls_residual_fwd(const void* A, int lda, const void* W, int ldw, const float* bias,
                                    const float* gamma, const float* resid, float* out, int ldo, int M, int N, int K,
                                    apla_stream_t stream);
+/* The residual update above with one scale per group of rows_per_scale rows (stochastic depth, vit.py drop_path):
+ * out_f32[m,n] = resid_f32[m,n] + row_scale_f32[m / rows_per_scale] * gamma_f32[n] * (A . W^T + bias)   (gamma NULL = 1).
+ * rows_per_scale = N scales the token rows of an image, 1 scales one row per image (the CLS rows, row stride ldo).
+ * A scale of 1 gives apla_gemm_bias_ls_residual_fwd's bits.  The default (2-CTA) GEMM only: refused under
+ * APLA_GEMM_IMPL=1.  NULL A, W, resid, row_scale or out, an empty shape or rows_per_scale < 1 are refused. */
+int apla_gemm_bias_ls_residual_scaled_fwd(const void* A, int lda, const void* W, int ldw, const float* bias,
+                                          const float* gamma, const float* resid, const float* row_scale,
+                                          int rows_per_scale, float* out, int ldo, int M, int N, int K,
+                                          apla_stream_t stream);
 /* The residual update above FOLLOWED BY the LayerNorm that reads it, in one launch:
  *   out_f32 = resid_f32 + gamma * (A . W^T + bias);  ln_out_bf16[M,N] = (out - mean) * rstd * ln_w + ln_b
  * i.e. vit.py:284 + the norm2 of vit.py:285 (projection), or vit.py:285 + the norm1 of the next block's vit.py:280 (fc2).
@@ -106,6 +115,15 @@ int apla_layernorm_bwd(const void* dy, int64_t ld_dy, const float* x, int64_t ld
                        void* sub, int64_t ld_sub, const int32_t* idx, int r, int r_pad, int rows, int D, float eps,
                        apla_stream_t stream);
 /* sub_bf16[t, j] = dy_bf16[t, idx[j]] (j < r), 0 (r <= j < r_pad). */
+/* apla_layernorm_bwd with dxb and sub of row t also multiplied by row_scale_f32[t / rows_per_scale] -- the
+ * stochastic-depth scale of the branch that reads them; dx_f32 (the residual-stream gradient) is not scaled.  A scale
+ * of 1 gives apla_layernorm_bwd's bits.  D a multiple of 128 only.  NULL dy, x, w, dx, dxb or row_scale, an empty shape
+ * or rows_per_scale < 1 are refused. */
+int apla_layernorm_bwd_scaled(const void* dy, int64_t ld_dy, const float* x, int64_t ldx, const float* w,
+                              const float* dres, int64_t ld_dres, float* dx, int64_t ld_dx, void* dxb, int64_t ld_dxb,
+                              const float* gamma, void* sub, int64_t ld_sub, const int32_t* idx, int r, int r_pad,
+                              const float* row_scale, int rows_per_scale, int rows, int D, float eps,
+                              apla_stream_t stream);
 int apla_gather_cols(const void* dy, int64_t ld, void* sub, int64_t ld_sub, const int32_t* idx, int r, int r_pad,
                      int rows, apla_stream_t stream);
 
@@ -332,6 +350,12 @@ typedef void* apla_engine_t;
 apla_engine_t apla_engine_create(int B, int N, int D, int H, int L, int hidden, int C, int patch, int img, int kpad,
                                  int r, int r_pad, int full_rows, float eps, float scale);
 void apla_engine_destroy(apla_engine_t e);
+/* Optional global buffers (NULL = unset): "hyper" f32[3] -- {lr, 1 - beta1^t, sqrt(1 - beta2^t)} read by the AdamW
+ * kernel instead of its arguments (replayable graphs); "drop_path" f32[L, 2, B] -- stochastic depth (vit.py drop_path):
+ * the scale (0 or 1/keep) of block l's attention (0) and MLP (1) branch for image b.  With it set, the training forward
+ * computes x_mid = x_in + s[l,0,b] * ls1(attn) and x_out = x_mid + s[l,1,b] * ls2(mlp) for the first n_img images, and the
+ * backward scales the bf16 gradient each branch reads by the same s (the fp32 residual gradient is not scaled); unset,
+ * the step runs exactly its launches without it.  The evaluation entries never read it. */
 int apla_engine_set_ptr(apla_engine_t e, const char* name, int block, void* p);
 /* Options (default in brackets): "infer_batch" [0] -- images per apla_engine_infer call (its workspace capacity);
  * "cls_only_last_block" [2] -- evaluate the per-token tail of the LAST block (projection,
