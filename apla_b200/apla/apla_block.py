@@ -24,8 +24,11 @@ Accepts `[B,N,D]` tensors (vit.py Block) and lists of `[b_i,N_i,D]` crops, which
 block-diagonally (dinov2 NestedTensorBlock.forward_nested; get_attn_bias_and_cat block.py:191-217).
 
 The residual stream is fp32 inside the node whatever the input dtype (what autocast keeps in fp32, SURVEY.md 8a); the
-output has the input's dtype.  CUDA (sm_100a) only, no fallback; dropout / drop-path / stochastic depth must be off
-(all shipped reference configs run them at 0).
+output has the input's dtype.  CUDA (sm_100a) only, no fallback.  Dropout must be off (all shipped reference configs run
+it at 0).  Stochastic depth (drop path, vit.py drop_path / timm `drop_path1` / `drop_path2`) runs on `[B,N,D]` tensors:
+in training mode the block calls its own drop-path modules on a ones tensor for the per-image branch scales, so it
+draws exactly the masks the unfused block draws, and the native calls scale each image's branch output by them
+(`apla_block_fwd_scaled` / `apla_block_bwd_scaled`).  Lists of crops with a nonzero drop-path rate are refused.
 """
 from __future__ import annotations
 
@@ -71,24 +74,28 @@ class _AplaBlockFn(torch.autograd.Function):
     with no Python between them."""
 
     @staticmethod
-    def forward(ctx, x, w1, b1, blk, cu_seqlens, seqlens):
+    def forward(ctx, x, w1, b1, blk, cu_seqlens, seqlens, scales):
         nat, x_in, T, num_seqs, max_len, (x_mid, x_out, qkv, ao, lse, ln_tmp, gelu_tmp) = _fwd_setup(blk, x, cu_seqlens,
                                                                                                     seqlens)
         dgelu = torch.empty(T, blk.mlp.fc1.out_features, device=x.device, dtype=torch.float16)
-        LIB.call("apla_block_fwd", ctypes.addressof(nat), ptr(x_in), ptr(x_mid), ptr(x_out), ptr(ln_tmp), ptr(qkv), ptr(ao),
-                 ptr(lse), ptr(dgelu), ptr(gelu_tmp), ptr(cu_seqlens), num_seqs, max_len, T, stream())
+        args = (ctypes.addressof(nat), ptr(x_in), ptr(x_mid), ptr(x_out), ptr(ln_tmp), ptr(qkv), ptr(ao), ptr(lse),
+                ptr(dgelu), ptr(gelu_tmp), ptr(cu_seqlens), num_seqs, max_len, T)
+        if scales is None:
+            LIB.call("apla_block_fwd", *args, stream())
+        else:
+            LIB.call("apla_block_fwd_scaled", *args, ptr(scales), T // x.shape[0], stream())
         ctx.blk, ctx.nat, ctx.refs = blk, nat, blk._nat_refs      # the struct points into these tensors
         blk._dyb_stash = None                                     # (see backward: nothing survives from the last step)
         ctx.geom = (num_seqs, max_len, cu_seqlens)
         ctx.x_dtype, ctx.x_shape = x.dtype, x.shape
-        ctx.save_for_backward(x_in, x_mid, qkv, ao, lse, dgelu)
+        ctx.save_for_backward(x_in, x_mid, qkv, ao, lse, dgelu, scales)
         return x_out.view(x.shape).to(x.dtype)
 
     @staticmethod
     def backward(ctx, dy):
         blk, nat = ctx.blk, ctx.nat
         at = blk.attn
-        x_in, x_mid, qkv, ao, lse, dgelu = ctx.saved_tensors
+        x_in, x_mid, qkv, ao, lse, dgelu, scales = ctx.saved_tensors
         num_seqs, max_len, cu = ctx.geom
         D, H, Hd, r = at.dim, at.num_heads, blk.mlp.fc1.out_features, at.partial_size
         want_w = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
@@ -102,12 +109,14 @@ class _AplaBlockFn(torch.autograd.Function):
         # written.  That block writes it from its last LayerNorm backward instead and leaves it here -- accepted only if
         # `dy` IS that gradient, untouched: same storage, same version counter (autograd accumulating a second consumer's
         # gradient into it, in place or not, changes one of the two).
+        # With drop path, a block needs bf16(s1 * gamma2 * dy), whose per-image scale s1 the block behind it cannot know:
+        # it forms that itself (a row-scaled cast), and the block behind writes no hand-over for it.
         stash, blk._dyb_stash = getattr(blk, "_dyb_stash", None), None
-        dyb_ready = int(stash is not None and stash[0] == dx_out.data_ptr() and stash[1] == dx_out._version
-                        and stash[2] == T and stash[3].device == dev)
+        dyb_ready = int(scales is None and stash is not None and stash[0] == dx_out.data_ptr()
+                        and stash[1] == dx_out._version and stash[2] == T and stash[3].device == dev)
         dyb = stash[3] if dyb_ready else torch.empty(T, D, device=dev, dtype=bf)
         front = blk._front_ref() if getattr(blk, "_front_ref", None) is not None else None
-        chain = bool(want_x and front is not None and _CHAIN and front.attn.dim == D)
+        chain = bool(want_x and front is not None and _CHAIN and front.attn.dim == D and not front._drop_path_active())
         dyb_front = torch.empty(T, D, device=dev, dtype=bf) if chain else None
         g_front = front._mlp_working_set(dev)["g2"] if chain else None
         dh = torch.empty(T, Hd, device=dev, dtype=bf)
@@ -121,14 +130,17 @@ class _AplaBlockFn(torch.autograd.Function):
         if want_w:
             dw1 = torch.empty(r, D, device=dev, dtype=f32)       # zeroed by the library
             db1 = torch.empty(r, device=dev, dtype=f32)
-        LIB.call("apla_block_bwd", ctypes.addressof(nat), ptr(dx_out), ptr(x_in), ptr(x_mid), ptr(qkv), ptr(ao), ptr(lse),
-                 ptr(dgelu), ptr(dx_mid), ptr(dx_mid) if want_x else None, ptr(dyb), ptr(dh), ptr(dln), ptr(dsub), ptr(d_ao),
-                 ptr(delta), ptr(dqkv), ptr(dw1), ptr(db1), ptr(cu), num_seqs, max_len, T, dyb_ready, ptr(dyb_front),
-                 ptr(g_front), stream())
+        args = (ctypes.addressof(nat), ptr(dx_out), ptr(x_in), ptr(x_mid), ptr(qkv), ptr(ao), ptr(lse), ptr(dgelu),
+                ptr(dx_mid), ptr(dx_mid) if want_x else None, ptr(dyb), ptr(dh), ptr(dln), ptr(dsub), ptr(d_ao), ptr(delta),
+                ptr(dqkv), ptr(dw1), ptr(db1), ptr(cu), num_seqs, max_len, T, dyb_ready, ptr(dyb_front), ptr(g_front))
+        if scales is None:
+            LIB.call("apla_block_bwd", *args, stream())
+        else:
+            LIB.call("apla_block_bwd_scaled", *args, ptr(scales), T // ctx.x_shape[0], stream())
         dx = dx_mid.view(ctx.x_shape).to(ctx.x_dtype) if want_x else None
         if chain and dx.data_ptr() == dx_mid.data_ptr():
             front._dyb_stash = (dx_mid.data_ptr(), dx._version, T, dyb_front)
-        return dx, dw1, db1, None, None, None
+        return dx, dw1, db1, None, None, None, None
 
 
 def _gamma_of(ls) -> Optional[torch.Tensor]:
@@ -226,35 +238,80 @@ class FusedAplaBlock(nn.Module):
             self._nat, self._nat_key, self._nat_refs = nat, key, (ws, ms)
         return self._nat
 
-    def _check(self, x):
+    def _drop_path_modules(self):
+        """The (attention, MLP) branch's drop-path module: timm's / DINOv2's `drop_path1` / `drop_path2`, else the one
+        `drop_path` the reference's Block calls for both branches (vit.py); None where the block has none."""
+        one = getattr(self, "drop_path", None)
+        return getattr(self, "drop_path1", one), getattr(self, "drop_path2", one)
+
+    def _drop_path_active(self) -> bool:
+        return self.training and any(_drop_rate(m) > 0 for m in self._drop_path_modules())
+
+    def _branch_scales(self, x) -> Optional[torch.Tensor]:
+        """fp32 [2, B] per-image scales of the attention (row 0) and MLP (row 1) branch, or None when nothing is drawn
+        (eval mode, rate 0, nn.Identity).  Each comes from the branch's own drop-path module applied to ones(B, 1, 1) in
+        the dtype of the reference's branch output, attention branch first: the CUDA generator advances exactly as in the
+        unfused block, so the same seed gives the same masks whatever the DropPath implementation."""
+        if not self._drop_path_active():
+            return None
+        # dtypes of the branch outputs the reference drops: attn(norm1(x)) has x's dtype, the MLP's Linear output
+        # autocast's when it is on; LayerScale's gamma promotes either
+        g1, g2 = _gamma_of(self.ls1), _gamma_of(self.ls2)
+        dt_attn = x.dtype if g1 is None else torch.promote_types(x.dtype, g1.dtype)
+        dt_mlp = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else torch.promote_types(x.dtype,
+                                                                                                                 dt_attn)
+        dt_mlp = dt_mlp if g2 is None else torch.promote_types(dt_mlp, g2.dtype)
+        B = x.shape[0]
+        rows = []
+        for mod, dt in zip(self._drop_path_modules(), (dt_attn, dt_mlp)):
+            ones = torch.ones(B, 1, 1, device=x.device, dtype=dt)
+            rows.append((mod(ones) if _drop_rate(mod) > 0 else ones).reshape(B).to(torch.float32))
+        return torch.stack(rows)
+
+    def _check(self, x, crops: bool = False):
+        if self.training:
+            at = self.attn
+            drops = {"attn.attn_drop": at.attn_drop.p, "attn.proj_drop": at.proj_drop.p,
+                     "mlp.drop": _drop_rate(getattr(self.mlp, "drop", None))}
+            bad = [f"{k}={p}" for k, p in drops.items() if p > 0]
+            if bad:
+                raise RuntimeError(f"fused APLA block supports dropout rate 0 only (got {', '.join(bad)}; all shipped "
+                                   "reference configs use 0)")
+            if self.sample_drop_ratio > 0.1:
+                raise RuntimeError(f"fused APLA block: sample_drop_ratio={self.sample_drop_ratio} > 0.1 selects DINOv2's "
+                                   "batch-subset stochastic depth, which is not supported (per-image drop path is)")
+            if crops and self._drop_path_active():
+                raise RuntimeError("fused APLA block: drop path on a list of crops (DINOv2's batch-subset stochastic depth "
+                                   "of forward_nested) is not supported; drop path runs on dense [B, N, D] input only")
+            if self.attn.dim % 128 and self._drop_path_active():
+                raise RuntimeError(f"fused APLA block: drop path needs an embedding width that is a multiple of 128 (the "
+                                   f"row-scaled LayerNorm backward), got {self.attn.dim}; set the drop-path rate to 0")
         if not x.is_cuda:
             raise RuntimeError("apla_b200.FusedAplaBlock runs on CUDA (sm_100a) only; there is no CPU fallback")
         require_device()
-        if self.training:
-            at = self.attn
-            rates = [at.attn_drop.p, at.proj_drop.p, _drop_rate(getattr(self.mlp, "drop", None)), self.sample_drop_ratio]
-            rates += [_drop_rate(getattr(self, n, None)) for n in ("drop_path", "drop_path1", "drop_path2")]
-            if any(p > 0 for p in rates):
-                raise RuntimeError("fused APLA block supports dropout / drop-path rate 0 only "
-                                   "(all shipped reference configs use 0)")
         for p in (self.norm1.weight, self.norm2.weight, self.mlp.fc1.weight, self.mlp.fc2.weight):
             if p.requires_grad:
                 raise RuntimeError("fused APLA block computes weight gradients for proj_weight1 / proj_bias1 only; "
                                    "norm / MLP parameters must be frozen (build_apla's freeze policy)")
 
-    def _run_fused(self, x, cu=None, seqlens=None):
+    def _run_fused(self, x, cu=None, seqlens=None, scales=None):
         at = self.attn
         if not torch.is_grad_enabled() or not (x.requires_grad or at.proj_weight1.requires_grad
                                                 or at.proj_bias1.requires_grad):
-            return self._run_infer(x, cu, seqlens)      # autograd would record nothing: keep nothing for backward
-        return _AplaBlockFn.apply(x, at.proj_weight1, at.proj_bias1, self, cu, seqlens)
+            return self._run_infer(x, cu, seqlens, scales)      # autograd would record nothing: keep nothing for backward
+        return _AplaBlockFn.apply(x, at.proj_weight1, at.proj_bias1, self, cu, seqlens, scales)
 
-    def _run_infer(self, x, cu, seqlens):
+    def _run_infer(self, x, cu, seqlens, scales=None):
         """`apla_block_fwd_infer`: the forward of _AplaBlockFn, bit for bit, without its saved tensors (lse is scratch,
-        fc1 writes no GELU derivative).  x_out is a buffer of its own: x_in may be the caller's tensor."""
+        fc1 writes no GELU derivative).  x_out is a buffer of its own: x_in may be the caller's tensor.  A training-mode
+        block drops branches here too (`scales`), as the reference's Block does under torch.no_grad()."""
         nat, x_in, T, num_seqs, max_len, (x_mid, x_out, qkv, ao, lse, ln_tmp, gelu_tmp) = _fwd_setup(self, x, cu, seqlens)
-        LIB.call("apla_block_fwd_infer", ctypes.addressof(nat), ptr(x_in), ptr(x_mid), ptr(x_out), ptr(ln_tmp), ptr(qkv),
-                 ptr(ao), ptr(lse), ptr(gelu_tmp), ptr(cu), num_seqs, max_len, T, stream())
+        args = (ctypes.addressof(nat), ptr(x_in), ptr(x_mid), ptr(x_out), ptr(ln_tmp), ptr(qkv), ptr(ao), ptr(lse),
+                ptr(gelu_tmp), ptr(cu), num_seqs, max_len, T)
+        if scales is None:
+            LIB.call("apla_block_fwd_infer", *args, stream())
+        else:
+            LIB.call("apla_block_fwd_infer_scaled", *args, ptr(scales), T // x.shape[0], stream())
         return x_out.view(x.shape).to(x.dtype)
 
     def _attention(self, x):
@@ -284,11 +341,11 @@ class FusedAplaBlock(nn.Module):
             return self._attention(x_or_x_list)
         if isinstance(x_or_x_list, torch.Tensor):
             self._check(x_or_x_list)
-            return self._run_fused(x_or_x_list)
+            return self._run_fused(x_or_x_list, scales=self._branch_scales(x_or_x_list))
         xs: Sequence[torch.Tensor] = list(x_or_x_list)
         if not xs:
             raise AssertionError("empty crop list")
-        self._check(xs[0])
+        self._check(xs[0], crops=True)
         D = xs[0].shape[-1]
         seqlens: List[int] = []
         for t in xs:

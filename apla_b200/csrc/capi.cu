@@ -130,6 +130,14 @@ int apla_ls_cast(const float* x, int64_t ldx, const float* gamma, void* out, int
                  apla_stream_t stream) {
   return ls_cast(x, ldx, gamma, out, ldo, rows, D, S(stream));
 }
+int apla_ls_cast_scaled(const float* x, int64_t ldx, const float* gamma, void* out, int64_t ldo, const float* row_scale,
+                        int rows_per_scale, int rows, int D, apla_stream_t stream) {
+  if (!x || !out || !row_scale) {
+    set_error("apla_ls_cast_scaled: null x, out or row_scale");
+    return 1;
+  }
+  return ls_cast(x, ldx, gamma, out, ldo, rows, D, S(stream), row_scale, rows_per_scale);
+}
 
 int apla_attn_fwd(const void* qkv, void* out, float* lse, const int32_t* cu_seqlens, int num_seqs, int max_seqlen,
                   int total_tokens,

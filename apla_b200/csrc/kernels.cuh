@@ -80,8 +80,9 @@ int layernorm_bwd(const void* dy, int64_t ld_dy, const float* x, int64_t ldx, co
                   const float* row_scale = nullptr, int rows_per_scale = 1);
 int gather_cols(const void* dy, int64_t ld, void* sub, int64_t ld_sub, const int* idx, int r, int r_pad, int rows,
                 cudaStream_t stream);
+// row_scale set: row t is also scaled by row_scale[t / rows_per_scale]
 int ls_cast(const float* x, int64_t ldx, const float* gamma, void* out, int64_t ldo, int rows, int D,
-            cudaStream_t stream);
+            cudaStream_t stream, const float* row_scale = nullptr, int rows_per_scale = 1);
 int colsum(const void* a, int64_t ld, int rows, int n, float* out, const int* rowmap, cudaStream_t stream);
 int patchify(const float* img, void* out, int B, int S, int p, int kpad, cudaStream_t stream);
 int assemble_tokens(const void* patch, const float* cls, const float* pos, float* x, int B, int P, int D,

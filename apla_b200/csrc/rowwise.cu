@@ -255,9 +255,13 @@ __global__ void gather_cols_kernel(const __nv_bfloat16* __restrict__ dy, int64_t
 }
 
 // out_bf16[t, d] = gamma[d] * x_f32[t, d] (gamma NULL = 1): LayerScale backward + down-cast of a residual gradient that
-// arrives from outside the fused chain (autograd handing the block-level Function its dY); 4 elements per thread
-__global__ void ls_cast_kernel(const float* __restrict__ x, int64_t ldx, const float* __restrict__ gamma,
-                               __nv_bfloat16* __restrict__ out, int64_t ldo, int rows, int D4) {
+// arrives from outside the fused chain (autograd handing the block-level Function its dY); 4 elements per thread.
+// kScaled (ls_cast_scaled_kernel): also multiplied by the row's scale row_scale[t / rows_per_scale] -- the
+// stochastic-depth mask of the MLP branch that reads the result.
+template <bool kScaled>
+__device__ __forceinline__ void ls_cast_elem(const float* __restrict__ x, int64_t ldx, const float* __restrict__ gamma,
+                                             __nv_bfloat16* __restrict__ out, int64_t ldo, int rows, int D4,
+                                             const float* __restrict__ row_scale, int rows_per_scale) {
   const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= int64_t(rows) * D4) return;
   const int row = int(i / D4), c = int(i % D4) * 4;
@@ -266,11 +270,26 @@ __global__ void ls_cast_kernel(const float* __restrict__ x, int64_t ldx, const f
     const float4 g = __ldg(reinterpret_cast<const float4*>(gamma + c));
     v.x *= g.x; v.y *= g.y; v.z *= g.z; v.w *= g.w;
   }
+  if constexpr (kScaled) {
+    const float s = __ldg(row_scale + row / rows_per_scale);
+    v.x *= s; v.y *= s; v.z *= s; v.w *= s;
+  }
   __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
   uint2 pk;
   pk.x = *reinterpret_cast<uint32_t*>(&lo);
   pk.y = *reinterpret_cast<uint32_t*>(&hi);
   *reinterpret_cast<uint2*>(out + row * ldo + c) = pk;
+}
+
+__global__ void ls_cast_kernel(const float* __restrict__ x, int64_t ldx, const float* __restrict__ gamma,
+                               __nv_bfloat16* __restrict__ out, int64_t ldo, int rows, int D4) {
+  ls_cast_elem<false>(x, ldx, gamma, out, ldo, rows, D4, nullptr, 1);
+}
+
+__global__ void ls_cast_scaled_kernel(const float* __restrict__ x, int64_t ldx, const float* __restrict__ gamma,
+                                      __nv_bfloat16* __restrict__ out, int64_t ldo, int rows, int D4,
+                                      const float* __restrict__ row_scale, int rows_per_scale) {
+  ls_cast_elem<true>(x, ldx, gamma, out, ldo, rows, D4, row_scale, rows_per_scale);
 }
 
 // column sums of a bf16 [rows, n] matrix -> fp32 out[map(j)] (+=): bias gradient of the trainable rows
@@ -491,11 +510,17 @@ int gather_cols(const void* dy, int64_t ld, void* sub, int64_t ld_sub, const int
 }
 
 int ls_cast(const float* x, int64_t ldx, const float* gamma, void* out, int64_t ldo, int rows, int D,
-            cudaStream_t stream) {
+            cudaStream_t stream, const float* row_scale, int rows_per_scale) {
   APLA_CHECK(rows > 0 && D > 0 && D % 4 == 0 && ldx % 4 == 0 && ldo % 4 == 0, "ls_cast: bad shape rows=%d D=%d", rows, D);
   const int64_t total = int64_t(rows) * (D / 4);
-  ls_cast_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(x, ldx, gamma, reinterpret_cast<__nv_bfloat16*>(out),
-                                                                      ldo, rows, D / 4);
+  if (row_scale) {
+    APLA_CHECK(rows_per_scale >= 1, "ls_cast: rows_per_scale=%d must be >= 1", rows_per_scale);
+    ls_cast_scaled_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(
+        x, ldx, gamma, reinterpret_cast<__nv_bfloat16*>(out), ldo, rows, D / 4, row_scale, rows_per_scale);
+  } else {
+    ls_cast_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(
+        x, ldx, gamma, reinterpret_cast<__nv_bfloat16*>(out), ldo, rows, D / 4);
+  }
   APLA_CUDA(cudaGetLastError());
   count_launch();
   return 0;

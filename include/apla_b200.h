@@ -131,6 +131,11 @@ int apla_gather_cols(const void* dy, int64_t ld, void* sub, int64_t ld_sub, cons
  * gradient entering the fused block from autograd (Block.forward vit.py:279-288 seen from its output). */
 int apla_ls_cast(const float* x, int64_t ldx, const float* gamma, void* out, int64_t ldo, int rows, int D,
                  apla_stream_t stream);
+/* apla_ls_cast with row t also multiplied by row_scale_f32[t / rows_per_scale]: the gradient a block's MLP branch reads
+ * under stochastic depth, bf16(s1 * gamma2 * dx_out).  A scale of 1 gives apla_ls_cast's bits.  NULL x, out or
+ * row_scale, a bad shape or rows_per_scale < 1 are refused. */
+int apla_ls_cast_scaled(const float* x, int64_t ldx, const float* gamma, void* out, int64_t ldo, const float* row_scale,
+                        int rows_per_scale, int rows, int D, apla_stream_t stream);
 
 /* --- attention ------------------------------------------------------------------------------------------ */
 /* out_bf16[T, H*64] = softmax(scale * q k^T) v per sequence and head; lse_f32[T, H] saved for backward.
@@ -340,6 +345,29 @@ int apla_block_bwd(const apla_block_weights* w, const float* dx_out, const float
                    void* dyb, void* dh, void* dln, void* dsub, void* d_ao, float* delta, void* dqkv, float* dw1,
                    float* db1, const int32_t* cu_seqlens, int num_seqs, int max_seqlen, int T, int dyb_ready,
                    void* dyb_prev, const float* gamma_prev, apla_stream_t stream);
+/* Stochastic depth (vit.py drop_path): the three calls above with branch_scale f32[2, B], B = T / rows_per_scale images
+ * of rows_per_scale token rows each (rows_per_scale = N for dense [B, N, D] input).  branch_scale[0, b] (attention) and
+ * branch_scale[1, b] (MLP) multiply image b's branch output: x_mid = x_in + s0 * ls1(attn), x_out = x_mid + s1 * ls2(mlp)
+ * (EPI_RESID_SCALED).  The backward scales the bf16 gradient each branch reads by the same s -- dyb = bf16(s1 * g2 *
+ * dx_out) (row-scaled ls_cast) and the LayerNorm-2 backward's dyb / dsub by s0 -- and not the fp32 residual gradients.
+ * A block with scales forms its own dyb: dyb_ready must be 0 (a hand-over carries no scale).  branch_scale NULL: the
+ * unscaled call, same launches and arguments.  rows_per_scale < 1, or T not a multiple of it with scales, is refused.
+ * The scaled backward needs D a multiple of 128 (the row-scaled LayerNorm backward) and refuses other widths before
+ * any launch; the scaled forwards take any width the unscaled ones take. */
+int apla_block_fwd_scaled(const apla_block_weights* w, const float* x_in, float* x_mid, float* x_out, void* ln_tmp,
+                          void* qkv, void* ao, float* lse, void* dgelu, void* gelu_tmp, const int32_t* cu_seqlens,
+                          int num_seqs, int max_seqlen, int T, const float* branch_scale, int rows_per_scale,
+                          apla_stream_t stream);
+int apla_block_fwd_infer_scaled(const apla_block_weights* w, const float* x_in, float* x_mid, float* x_out,
+                                void* ln_tmp, void* qkv, void* ao, float* lse_tmp, void* gelu_tmp,
+                                const int32_t* cu_seqlens, int num_seqs, int max_seqlen, int T,
+                                const float* branch_scale, int rows_per_scale, apla_stream_t stream);
+int apla_block_bwd_scaled(const apla_block_weights* w, const float* dx_out, const float* x_in, const float* x_mid,
+                          const void* qkv, const void* ao, const float* lse, const void* dgelu, float* dx_mid,
+                          float* dx_in, void* dyb, void* dh, void* dln, void* dsub, void* d_ao, float* delta, void* dqkv,
+                          float* dw1, float* db1, const int32_t* cu_seqlens, int num_seqs, int max_seqlen, int T,
+                          int dyb_ready, void* dyb_prev, const float* gamma_prev, const float* branch_scale,
+                          int rows_per_scale, apla_stream_t stream);
 
 /* --- step engine: the whole fine-tune step as one native call sequence ------------------------------------ */
 /* Replaces Trainer.global_step's device work (src/defaults/trainer.py:106-138): Classifier.forward
